@@ -133,6 +133,31 @@ int prb_last_kernel_ms(prb_handle* h, float* ik_ms, float* step_ms);
  * thread-per-env solver launches of the most recent step */
 int prb_last_tier_ms(prb_handle* h, float* setup_ms, float* pgs_ms);
 
+/* Camera images of every env (the reference's calc_state 'img', environments.py:841-845, and its gripper camera,
+ * :33-49).  Every collider is drawn as the box it is in the compiled model, coloured from col_rgb_host ([n_col,3] in
+ * [0,1]: colours are not part of prb_model) and shaded rgb = clamp(colour (ambient + diffuse max(0, n.l)), 0, 1)
+ * with n the world normal of the face hit; no shadows.  view / proj are column-major 4x4 matrices in the layout
+ * PyBullet's computeViewMatrix* / computeProjectionMatrixFOV return; proj must be a perspective projection
+ * (clip w = -z_eye) and view a rigid transform.  Pixel (i, j), row 0 at the top, is the ray through NDC
+ * (2(j+0.5)/W-1, 1-2(i+0.5)/H). */
+typedef struct prb_camera {
+  int32_t width, height;   /* 1..1024 */
+  int32_t attach;          /* 0: view maps world to eye; 1: view maps the end-effector site frame to eye (gripper camera) */
+  float view[16];
+  float proj[16];
+  float light_dir[3];      /* towards the light, world frame; normalised by the library */
+  float ambient, diffuse;
+  float background[3];     /* colour of pixels that hit nothing */
+} prb_camera;
+
+/* Renders the current state of all envs: rgb_dev uint8 [N,H,W,3]; depth_dev float [N,H,W] eye-space depth in metres
+ * (far plane where nothing is hit) and seg_dev int32 [N,H,W] collider index (-1 where nothing is hit) are optional
+ * (NULL).  Reads the state only: no simulation state or step output changes.  Asynchronous on `stream`. */
+int prb_render(prb_handle* h, const prb_camera* cam, const float* col_rgb_host, uint8_t* rgb_dev, float* depth_dev,
+               int32_t* seg_dev, void* stream);
+/* Pixel-box slab tests prb_render has run since creation (after tile culling; for reports).  Synchronises the device. */
+int64_t prb_render_box_tests(prb_handle* h);
+
 /* Number of kernels launched by this handle since creation (bench.py reports it). */
 int64_t prb_launch_count(prb_handle* h);
 /* Env steps (since creation; a reset counts as one) in which a contact had to be dropped because the per-env

@@ -13,6 +13,7 @@
 #include <thread>
 #include <vector>
 #include "prb_reset.cuh"
+#include "prb_render.cuh"
 
 struct prb_handle {
   DevModel hm;
@@ -56,6 +57,7 @@ struct prb_handle {
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   cudaEvent_t evk[64];             // per-launch events of the most recent step (timing mode)
   int n_evk = 0;
+  unsigned long long* render_tests = nullptr;   // pixel-box tests of prb_render (allocated by the first render)
   std::string err;
 };
 
@@ -344,6 +346,7 @@ int prb_destroy(prb_handle* h) {
   if (h->side_free) cudaStreamDestroy(h->side_free);
   if (h->ev_join_free) cudaEventDestroy(h->ev_join_free);
   cudaFree(h->hbuf); cudaFree(h->heavy_cnt);
+  if (h->render_tests) cudaFree(h->render_tests);
   for (int i = 0; i < 3; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   if (h->ev[0]) for (int i = 0; i < 64; i++) cudaEventDestroy(h->evk[i]);
   }
@@ -552,6 +555,36 @@ int prb_step_host(prb_handle* h, const float* action_host, float* out_host, void
   for (int t = 0; t < T; t++) CK(h, werr[t]);
   CK(h, cudaStreamSynchronize(s));
   return PRB_OK;
+}
+
+int prb_render(prb_handle* h, const prb_camera* cam, const float* col_rgb_host, uint8_t* rgb_dev, float* depth_dev,
+               int32_t* seg_dev, void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!cam || !col_rgb_host || !rgb_dev) { h->err = "prb_render: camera, colours and rgb_dev are required"; return PRB_ERR_INVALID; }
+  RenderParams P;
+  const std::string why = render_params(*cam, col_rgb_host, h->hm.n_col, &P);
+  if (!why.empty()) { h->err = "prb_render: " + why; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (!h->render_tests) {
+    CK(h, cudaMalloc(&h->render_tests, sizeof(unsigned long long)));
+    CK(h, cudaMemsetAsync(h->render_tests, 0, sizeof(unsigned long long), s));
+  }
+  // one block per env; the kernel indexes pixels in 64 bits (65 536 envs x 1024 x 1024 x 3 bytes exceeds 2^32)
+  prb_render_kernel<<<h->N, 32 * RENDER_WARPS, 0, s>>>(h->dm, h->state, P, rgb_dev, depth_dev, seg_dev, h->render_tests);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  return PRB_OK;
+}
+
+int64_t prb_render_box_tests(prb_handle* h) {
+  if (!h) return -1;
+  if (!h->render_tests) return 0;
+  DevGuard guard(h->device);
+  unsigned long long v = 0;
+  if (cudaDeviceSynchronize() != cudaSuccess) return -1;
+  if (cudaMemcpy(&v, h->render_tests, sizeof(v), cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
+  return (int64_t)v;
 }
 
 int64_t prb_launch_count(prb_handle* h) { return h ? h->launches : 0; }

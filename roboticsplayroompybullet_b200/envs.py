@@ -14,12 +14,17 @@ Two calling styles: numpy in / numpy out (`step`), which goes through host buffe
 reference user would (H2D of actions, D2H of the whole observation block every step), and
 `step_device` for learners that keep everything on the GPU (torch tensors, zero-copy views of the
 library's buffers).
+
+With record_images=True every observation also carries 'img' (environments.py:841-845): a uint8 [N,H,W,3] frame of
+`camera` (default: camera.default_camera) rendered on the GPU by prb_render after the step.  render() / render_device()
+draw any other camera (e.g. camera.gripper_camera) with optional depth and segmentation.
 """
 import ctypes
 
 import numpy as np
 
 from . import lib as _lib
+from .camera import camera_struct, default_camera, default_palette
 from .model import ACTION_VARIANTS, ENV_KINDS, action_dim, load_model
 
 OUT_KEYS = ['obs_quat', 'achieved_goal', 'desired_goal', 'controllable_achieved_goal', 'full_positional_state',
@@ -39,7 +44,8 @@ class _DevArray:
 class VecPlayEnv:
     env_id = None
 
-    def __init__(self, env_id=None, num_envs=1, device=0, seed=1234, env_offset=0, sparse=True, model=None):
+    def __init__(self, env_id=None, num_envs=1, device=0, seed=1234, env_offset=0, sparse=True, model=None,
+                 record_images=False, camera=None):
         import torch  # device memory / streams only
         self.torch = torch
         env_id = env_id or self.env_id
@@ -97,13 +103,39 @@ class VecPlayEnv:
         self.sparse = sparse
         self.h2d_bytes_per_step = N * self.action_dim * 4
         self.d2h_bytes_per_step = self.out_floats * 4
+        # camera images (calc_state 'img'): rendered only when asked for; colours per collider, [n_col, 3] in [0, 1]
+        self.record_images = bool(record_images)
+        self.camera = camera if camera is not None else default_camera(m)
+        self.palette = default_palette(m)
+        self._img = None
+        if self.record_images:
+            self._img = torch.empty((N, self.camera.height, self.camera.width, 3), dtype=torch.uint8, device=self.device)
 
     # ------------------------------------------------------------------ helpers
     def _stream(self):
         return ctypes.c_void_p(self.torch.cuda.current_stream(self.device).cuda_stream)
 
     def _obs_dev(self):
-        return {k: self.dev[k] for k in OBS_KEYS}
+        d = {k: self.dev[k] for k in OBS_KEYS}
+        if self.record_images:
+            d['img'] = self._render_img()
+        return d
+
+    def _render_img(self):
+        """'img' of the current state into the handle's frame buffer (allocated again if self.camera changed size)."""
+        cam = self.camera
+        if self._img is None or self._img.shape[1:3] != (cam.height, cam.width):
+            self._img = self.torch.empty((self.num_envs, cam.height, cam.width, 3), dtype=self.torch.uint8, device=self.device)
+        self._render(cam, self._img)
+        return self._img
+
+    def _render(self, camera, rgb, depth=None, seg=None):
+        cs = camera_struct(camera)
+        pal = np.ascontiguousarray(self.palette, np.float32)
+        assert pal.shape == (int(self.model['n_col']), 3), 'palette must be [n_col, 3]'
+        ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        _lib.check(self.L, self._h, self.L.prb_render(self._h, ctypes.byref(cs), ctypes.c_void_p(pal.ctypes.data), ptr(rgb),
+                                                     ptr(depth), ptr(seg), self._stream()))
 
     def _host_copy(self):
         """Fresh arrays for the caller (the reference returns copies, environments.py:850-855): ONE copy of the pinned result
@@ -115,7 +147,7 @@ class VecPlayEnv:
         c = c if c is not None else self._host_copy()
         d = {k: c[k] for k in OBS_KEYS}
         d['gripper_proprioception'] = d['gripper_proprioception'][:, 0].astype(np.int64)
-        d['img'] = None                                  # environments.py:844-845
+        d['img'] = self._img.cpu().numpy() if self.record_images else None    # environments.py:841-845
         return d
 
     def close(self):
@@ -194,6 +226,8 @@ class VecPlayEnv:
         r = c['reward'][:, 0]
         info = {'is_success': c['is_success'][:, 0].astype(np.int64), 'target_poses': c['target_poses']}
         done = np.zeros(self.num_envs, dtype=bool)       # environments.py:212: always False
+        if self.record_images:
+            self._render_img()
         return self._obs_host(c), r, done, info
 
     def reset_goal_pos(self, goal):
@@ -252,6 +286,29 @@ class VecPlayEnv:
                                                              ctypes.c_void_p(dgd.data_ptr()), agd.shape[0],
                                                              ctypes.c_void_p(out.data_ptr()), self._stream()))
         return out
+
+    # ------------------------------------------------------------------ camera images
+    def render_device(self, camera=None, depth=False, segmentation=False):
+        """Frame of the current state from `camera` (default: the env's camera): dict of CUDA tensors 'rgb' uint8
+        [N,H,W,3] and, when asked for, 'depth' float32 [N,H,W] (eye-space depth in metres, the far plane where nothing
+        is hit) and 'segmentation' int32 [N,H,W] (collider index, -1 where nothing is hit).  Asynchronous."""
+        cam = camera if camera is not None else self.camera
+        t, N, H, W = self.torch, self.num_envs, cam.height, cam.width
+        out = {'rgb': t.empty((N, H, W, 3), dtype=t.uint8, device=self.device)}
+        if depth:
+            out['depth'] = t.empty((N, H, W), dtype=t.float32, device=self.device)
+        if segmentation:
+            out['segmentation'] = t.empty((N, H, W), dtype=t.int32, device=self.device)
+        self._render(cam, out['rgb'], out.get('depth'), out.get('segmentation'))
+        return out
+
+    def render(self, camera=None, depth=False, segmentation=False):
+        """render_device() as numpy arrays."""
+        return {k: v.cpu().numpy() for k, v in self.render_device(camera, depth, segmentation).items()}
+
+    def render_box_tests(self):
+        """Pixel-box tests the renders of this handle have run (after tile culling)."""
+        return int(self.L.prb_render_box_tests(self._h))
 
     # ------------------------------------------------------------------ raw state (tests, checkpoints)
     def get_state(self):

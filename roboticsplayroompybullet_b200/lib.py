@@ -28,10 +28,17 @@ class PrbBuffers(ctypes.Structure):
                 [(n, ctypes.c_int32) for n in _INTS])
 
 
+class PrbCamera(ctypes.Structure):
+    _fields_ = [('width', ctypes.c_int32), ('height', ctypes.c_int32), ('attach', ctypes.c_int32),
+                ('view', ctypes.c_float * 16), ('proj', ctypes.c_float * 16), ('light_dir', ctypes.c_float * 3),
+                ('ambient', ctypes.c_float), ('diffuse', ctypes.c_float), ('background', ctypes.c_float * 3)]
+
+
 # every symbol include/prb.h declares (a CPU test checks the built library exports them all)
 SYMBOLS = ['prb_create', 'prb_destroy', 'prb_reset', 'prb_reset_rounds', 'prb_reset_to', 'prb_set_goal', 'prb_step', 'prb_observe', 'prb_substeps',
            'prb_get_buffers', 'prb_compute_reward', 'prb_get_state', 'prb_set_state', 'prb_step_host',
-           'prb_enable_kernel_timing', 'prb_last_kernel_ms', 'prb_last_tier_ms', 'prb_launch_count', 'prb_overflow_count', 'prb_debug_usage', 'prb_kernel_info', 'prb_last_error', 'prb_version']
+           'prb_enable_kernel_timing', 'prb_last_kernel_ms', 'prb_last_tier_ms', 'prb_launch_count', 'prb_overflow_count', 'prb_debug_usage', 'prb_kernel_info', 'prb_render', 'prb_render_box_tests', 'prb_last_error',
+           'prb_version']
 
 
 class PrbError(RuntimeError):
@@ -70,6 +77,9 @@ def load():
     L.prb_debug_usage.argtypes = [vp, vp]
     L.prb_overflow_count.restype = i64
     L.prb_kernel_info.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i32)]
+    L.prb_render.argtypes = [vp, ctypes.POINTER(PrbCamera), vp, vp, vp, vp, vp]
+    L.prb_render_box_tests.argtypes = [vp]
+    L.prb_render_box_tests.restype = i64
     L.prb_last_error.argtypes = [vp]
     L.prb_last_error.restype = ctypes.c_char_p
     L.prb_version.restype = ctypes.c_char_p
