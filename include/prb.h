@@ -158,6 +158,45 @@ int prb_render(prb_handle* h, const prb_camera* cam, const float* col_rgb_host, 
 /* Pixel-box slab tests prb_render has run since creation (after tile culling; for reports).  Synchronises the device. */
 int64_t prb_render_box_tests(prb_handle* h);
 
+/* Contact report: the contact points and forces of every env after a step, like PyBullet's getContactPoints() after
+ * stepSimulation().  Off by default; prb_enable_contacts(h, 1) allocates the report (the first time) and empties it.
+ * While enabled, prb_step, prb_step_host and prb_substeps (n >= 1) fill it with the contacts the LAST physics substep of
+ * the call solved; prb_reset, prb_reset_to and prb_set_state empty it (count 0) for every env whose state they change;
+ * prb_observe, prb_set_goal and prb_render leave it unchanged.  With PRB_PIPELINE=fused enabling fails (PRB_ERR_INVALID).
+ *
+ * Env e has count[e] (0..max_contacts = 64) contacts: those after manifold reduction (<= 4 per pair of collision
+ * objects), in the order the setup kernel generated them, which is the order the solver visits them (Bullet's).  For
+ * contact i < count[e], at [e, i] of each [N, 64] array and [e, i, :] of each [N, 64, 3] array:
+ *   collider_a, collider_b   collider indices of the model (the ids prb_render's segmentation uses); A is the pair's first
+ *                            collider (prb_model pair_a: the movable side of lowest body index)
+ *   position_on_a, _on_b     world, m; position_on_a = position_on_b + distance * normal_on_b
+ *   normal_on_b              unit, world, pointing from B towards A
+ *   distance                 m; negative: penetration
+ *   normal_force             normal impulse of the contact's row / dt, N, >= 0
+ *   lateral_friction_1, _2   friction impulses of its two rows / dt, N: signed force on A along lateral_friction_dir_1, _2
+ *   lateral_friction_dir_1, _2   the friction rows' directions (Bullet's btPlaneSpace1 of the normal)
+ * Entries i >= count[e] hold -1 (collider ids) and 0 (floats).  The torsional-friction impulse is not reported (PyBullet
+ * does not report it either).  That PyBullet reports applied impulse / time step as its forces, and the direction of
+ * its normal, are recalled from Bullet's sources, not verified against a PyBullet run. */
+typedef struct prb_contacts {
+  int32_t* count;                   /* [N] */
+  int32_t* collider_a;              /* [N,64] */
+  int32_t* collider_b;              /* [N,64] */
+  float* position_on_a;             /* [N,64,3] */
+  float* position_on_b;             /* [N,64,3] */
+  float* normal_on_b;               /* [N,64,3] */
+  float* distance;                  /* [N,64] */
+  float* normal_force;              /* [N,64] */
+  float* lateral_friction_1;        /* [N,64] */
+  float* lateral_friction_2;        /* [N,64] */
+  float* lateral_friction_dir_1;    /* [N,64,3] */
+  float* lateral_friction_dir_2;    /* [N,64,3] */
+  int32_t num_envs, max_contacts;
+} prb_contacts;
+int prb_enable_contacts(prb_handle* h, int32_t enable);
+/* Device pointers of the report (handle-owned; valid until prb_destroy).  Fails if the report was never enabled. */
+int prb_get_contacts(prb_handle* h, prb_contacts* out);
+
 /* Number of kernels launched by this handle since creation (bench.py reports it). */
 int64_t prb_launch_count(prb_handle* h);
 /* Env steps (since creation; a reset counts as one) in which a contact had to be dropped because the per-env

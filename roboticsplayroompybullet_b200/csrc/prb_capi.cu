@@ -14,6 +14,7 @@
 #include <vector>
 #include "prb_reset.cuh"
 #include "prb_render.cuh"
+#include "prb_contacts.cuh"
 
 struct prb_handle {
   DevModel hm;
@@ -58,6 +59,8 @@ struct prb_handle {
   cudaEvent_t evk[64];             // per-launch events of the most recent step (timing mode)
   int n_evk = 0;
   unsigned long long* render_tests = nullptr;   // pixel-box tests of prb_render (allocated by the first render)
+  float* crep = nullptr;           // contact report (prb_stream.cuh layout; allocated when first enabled)
+  int contacts = 0;                // 1: prb_step / prb_substeps refresh the contact report
   std::string err;
 };
 
@@ -87,6 +90,9 @@ struct DevGuard {
 // One env step (or n raw substeps).  Split pipeline: per substep one warp-per-env setup launch
 // (integrate previous solution + build rows) and the thread-per-env solver launches; a final setup
 // launch integrates the last solution and writes the observation.  No host synchronisation.
+// With the contact report enabled, a step of all envs (not a reset's masked settle steps) also fills the report from
+// its last substep: that substep's setup launch writes the contacts, its solvers write their impulses back, and one
+// prb_contact_report_kernel launch after the final setup launch writes the forces.
 template <int ND>
 static int launch_step(prb_handle* h, int nsub, int observe, cudaStream_t s, const unsigned char* active = nullptr,
                        const int* elist = nullptr, int n_list = 0) {
@@ -114,12 +120,15 @@ static int launch_step(prb_handle* h, int nsub, int observe, cudaStream_t s, con
     if (gcls[k] > want) gcls[k] = want;
   }
   const bool timed = h->timing != 0;
+  const bool report = h->contacts && active == nullptr && elist == nullptr && nsub > 0;
   for (int i = 0; i <= nsub; i++) {
+    const int wb = (report && i == nsub - 1) ? 1 : 0;
     int flags = (i > 0 ? SETUP_INTEGRATE : 0) | (i < nsub ? SETUP_BUILD : 0) | ((i == nsub && observe) ? SETUP_OBSERVE : 0);
     if (flags == 0) break;
     if (timed && h->n_evk < 62) CK(h, cudaEventRecord(h->evk[h->n_evk++], s));
     if (i < nsub) CK(h, cudaMemsetAsync(h->heavy_cnt, 0, 4 * ARM_NCLASS * sizeof(int), s));
-    prb_setup_kernel<ND><<<gs, bs, h->smem, s>>>(h->dm, h->state, h->sbuf, h->O, N, flags, h->hbuf, h->heavy_cnt, active, elist, n_list);
+    prb_setup_kernel<ND><<<gs, bs, h->smem, s>>>(h->dm, h->state, h->sbuf, h->O, N, flags, h->hbuf, h->heavy_cnt, active, elist, n_list,
+                                                    wb ? h->crep : nullptr);
     h->launches++;
     if (i < nsub) {
       if (timed && h->n_evk < 62) CK(h, cudaEventRecord(h->evk[h->n_evk++], s));
@@ -132,11 +141,11 @@ static int launch_step(prb_handle* h, int nsub, int observe, cudaStream_t s, con
         float4* hc = h->hbuf + arm_class_base(k, N);
         int* wc = h->heavy_cnt + 4 * k;
         switch (k) {                                      // envs per block = the record stride, a template constant
-          case 0: prb_pgs_arm_kernel<ND, false, arm_lanes(0)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k)); break;
-          case 1: prb_pgs_arm_kernel<ND, false, arm_lanes(1)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k)); break;
-          case 2: prb_pgs_arm_kernel<ND, false, arm_lanes(2)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k)); break;
-          case 3: prb_pgs_arm_kernel<ND, false, arm_lanes(3)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k)); break;
-          default: prb_pgs_arm_kernel<ND, true, arm_lanes(4)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k)); break;
+          case 0: prb_pgs_arm_kernel<ND, false, arm_lanes(0)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k), wb); break;
+          case 1: prb_pgs_arm_kernel<ND, false, arm_lanes(1)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k), wb); break;
+          case 2: prb_pgs_arm_kernel<ND, false, arm_lanes(2)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k), wb); break;
+          case 3: prb_pgs_arm_kernel<ND, false, arm_lanes(3)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k), wb); break;
+          default: prb_pgs_arm_kernel<ND, true, arm_lanes(4)><<<gcls[k], 32, smcls[k], h->side[k]>>>(h->dm, h->sbuf, hc, wc, arm_capq(k), arm_bufq(k), wb); break;
         }
         CK(h, cudaEventRecord(h->ev_join[k], h->side[k]));
       }
@@ -144,11 +153,11 @@ static int launch_step(prb_handle* h, int nsub, int observe, cudaStream_t s, con
       if (h->hm.n_free > 0) {
         if (h->free_side) {
           CK(h, cudaStreamWaitEvent(h->side_free, h->ev_fork, 0));
-          prb_pgs_free_kernel<<<gf, bp, PGS_SMEM_F, h->side_free>>>(h->dm, h->sbuf, N, active, elist, n_list);
+          prb_pgs_free_kernel<<<gf, bp, PGS_SMEM_F, h->side_free>>>(h->dm, h->sbuf, N, active, elist, n_list, wb);
           CK(h, cudaEventRecord(h->ev_join_free, h->side_free));
           CK(h, cudaStreamWaitEvent(s, h->ev_join_free, 0));
         } else {
-          prb_pgs_free_kernel<<<gf, bp, PGS_SMEM_F, s>>>(h->dm, h->sbuf, N, active, elist, n_list);
+          prb_pgs_free_kernel<<<gf, bp, PGS_SMEM_F, s>>>(h->dm, h->sbuf, N, active, elist, n_list, wb);
         }
       }
       for (int k = 0; k < ARM_NCLASS; k++) CK(h, cudaStreamWaitEvent(s, h->ev_join[k], 0));
@@ -156,6 +165,21 @@ static int launch_step(prb_handle* h, int nsub, int observe, cudaStream_t s, con
     }
   }
   if (timed && h->n_evk < 64) CK(h, cudaEventRecord(h->evk[h->n_evk++], s));
+  if (report) {
+    prb_contact_report_kernel<<<(N + CREP_WPB - 1) / CREP_WPB, 32 * CREP_WPB, 0, s>>>(h->crep, h->sbuf, h->hbuf, N, h->hm.params[P_DT],
+                                                                                    CREP_REPORT, nullptr);
+    h->launches++;
+  }
+  CK(h, cudaGetLastError());
+  return PRB_OK;
+}
+
+// prb_reset / prb_reset_to / prb_set_state: the report of the envs they change becomes empty (mask NULL: all envs)
+static int clear_contacts(prb_handle* h, const uint8_t* mask_dev, cudaStream_t s) {
+  if (!h->contacts) return PRB_OK;
+  prb_contact_report_kernel<<<(h->N + CREP_WPB - 1) / CREP_WPB, 32 * CREP_WPB, 0, s>>>(h->crep, h->sbuf, h->hbuf, h->N, h->hm.params[P_DT],
+                                                                                     CREP_CLEAR, mask_dev);
+  h->launches++;
   CK(h, cudaGetLastError());
   return PRB_OK;
 }
@@ -347,6 +371,7 @@ int prb_destroy(prb_handle* h) {
   if (h->ev_join_free) cudaEventDestroy(h->ev_join_free);
   cudaFree(h->hbuf); cudaFree(h->heavy_cnt);
   if (h->render_tests) cudaFree(h->render_tests);
+  if (h->crep) cudaFree(h->crep);
   for (int i = 0; i < 3; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   if (h->ev[0]) for (int i = 0; i < 64; i++) cudaEventDestroy(h->evk[i]);
   }
@@ -433,6 +458,8 @@ int prb_reset(prb_handle* h, const uint8_t* mask_dev, void* stream) {
   if (!h) return PRB_ERR_INVALID;
   DevGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
+  const int rc = clear_contacts(h, mask_dev, s);
+  if (rc != PRB_OK) return rc;
   return h->hm.nd == 12 ? reset_rounds<12>(h, mask_dev, s) : reset_rounds<9>(h, mask_dev, s);
 }
 
@@ -442,6 +469,8 @@ int prb_reset_to(prb_handle* h, const float* obs_dev, const uint8_t* mask_dev, i
   if (!h || !obs_dev) return PRB_ERR_INVALID;
   DevGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
+  const int rc = clear_contacts(h, mask_dev, s);
+  if (rc != PRB_OK) return rc;
   dim3 g((h->N + SetupCfg::WPB - 1) / SetupCfg::WPB), b(32 * SetupCfg::WPB);
   if (h->hm.nd == 12) prb_reset_to_kernel<12><<<g, b, h->smem, s>>>(h->dm, h->state, h->O, obs_dev, mask_dev, h->N, h->seed, h->env_offset, restore_env);
   else prb_reset_to_kernel<9><<<g, b, h->smem, s>>>(h->dm, h->state, h->O, obs_dev, mask_dev, h->N, h->seed, h->env_offset, restore_env);
@@ -497,7 +526,7 @@ int prb_set_state(prb_handle* h, const float* host_in) {
   CK(h, cudaDeviceSynchronize());
   CK(h, cudaMemcpy2D(h->state, sizeof(float) * M.state_stride, host_in, sizeof(float) * M.state_dim,
                      sizeof(float) * M.state_dim, h->N, cudaMemcpyHostToDevice));
-  return PRB_OK;
+  return clear_contacts(h, nullptr, nullptr);
 }
 
 int prb_step_host(prb_handle* h, const float* action_host, float* out_host, void* stream) {
@@ -585,6 +614,47 @@ int64_t prb_render_box_tests(prb_handle* h) {
   if (cudaDeviceSynchronize() != cudaSuccess) return -1;
   if (cudaMemcpy(&v, h->render_tests, sizeof(v), cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
   return (int64_t)v;
+}
+
+int prb_enable_contacts(prb_handle* h, int32_t enable) {
+  if (!h) return PRB_ERR_INVALID;
+  if (enable && h->fused) {
+    h->err = "prb_enable_contacts: PRB_PIPELINE=fused has no record stream to report contacts from";
+    return PRB_ERR_INVALID;
+  }
+  DevGuard guard(h->device);
+  if (enable && !h->contacts) {                    // off -> on: the report starts empty
+    const int64_t N = h->N;
+    if (!h->crep) CK(h, cudaMalloc(&h->crep, crep_words(N) * sizeof(float)));
+    CK(h, cudaDeviceSynchronize());
+    CK(h, cudaMemset(h->crep, 0, crep_words(N) * sizeof(float)));
+    CK(h, cudaMemset(crep_field(h->crep, N, CREP_COL_A), 0xff, 2 * N * SB_MAXCONTACT * sizeof(float)));    // collider ids -1
+    CK(h, cudaDeviceSynchronize());
+  }
+  h->contacts = enable ? 1 : 0;
+  return PRB_OK;
+}
+
+int prb_get_contacts(prb_handle* h, prb_contacts* out) {
+  if (!h || !out) return PRB_ERR_INVALID;
+  if (!h->crep) { h->err = "prb_get_contacts: the contact report was never enabled (prb_enable_contacts)"; return PRB_ERR_INVALID; }
+  float* c = h->crep;
+  const int64_t N = h->N;
+  out->count = crep_count(c, N);
+  out->collider_a = reinterpret_cast<int32_t*>(crep_field(c, N, CREP_COL_A));
+  out->collider_b = reinterpret_cast<int32_t*>(crep_field(c, N, CREP_COL_B));
+  out->position_on_a = crep_field(c, N, CREP_POS_A);
+  out->position_on_b = crep_field(c, N, CREP_POS_B);
+  out->normal_on_b = crep_field(c, N, CREP_NORMAL);
+  out->distance = crep_field(c, N, CREP_DIST);
+  out->normal_force = crep_field(c, N, CREP_FN);
+  out->lateral_friction_1 = crep_field(c, N, CREP_F1);
+  out->lateral_friction_2 = crep_field(c, N, CREP_F2);
+  out->lateral_friction_dir_1 = crep_field(c, N, CREP_DIR1);
+  out->lateral_friction_dir_2 = crep_field(c, N, CREP_DIR2);
+  out->num_envs = h->N;
+  out->max_contacts = SB_MAXCONTACT;
+  return PRB_OK;
 }
 
 int64_t prb_launch_count(prb_handle* h) { return h ? h->launches : 0; }

@@ -137,6 +137,32 @@ PRB_HD int arm_class_of(int tEnd) {
 #define DVW_SLIDE(s) (28 + (s))
 enum { K_STATIC = 0, K_FREE = 1, K_SLIDE = 2, K_ARM = 3 };
 
+// ---- contact report (prb_enable_contacts, include/prb.h): one allocation, field-major.  With NS = N * SB_MAXCONTACT and
+// s = e * SB_MAXCONTACT + i, scalar field f of contact i of env e is word f * NS + s; a 3-vector field takes three units,
+// [N, 64, 3] from word f * NS.  The int32 count [N] follows the 21 fields.  Between the setup launch that writes a
+// contact's geometry and prb_contact_report_kernel (prb_contacts.cuh), the words CREP_F1 / CREP_F2 of the contact hold the
+// 64-bit locator of its impulses: (float4 offset of the slot-0 record's quad +3 in the heavy allocation) << 1, or (q of the
+// compact record in the env's stream column) << 1 | 1.
+enum { CREP_COL_A = 0, CREP_COL_B = 1, CREP_POS_A = 2, CREP_POS_B = 5, CREP_NORMAL = 8, CREP_DIST = 11, CREP_FN = 12,
+       CREP_F1 = 13, CREP_F2 = 14, CREP_DIR1 = 15, CREP_DIR2 = 18, CREP_WORDS = 21 };
+PRB_HD size_t crep_words(int64_t N) { return (size_t)N * (CREP_WORDS * SB_MAXCONTACT + 1); }
+PRB_HD float* crep_field(float* crep, int64_t N, int f) { return crep + (size_t)f * N * SB_MAXCONTACT; }
+PRB_HD int* crep_count(float* crep, int64_t N) { return reinterpret_cast<int*>(crep_field(crep, N, CREP_WORDS)); }
+PRB_D void crep_geometry(float* crep, int N, int e, int i, int ca, int cb, v3 pa, v3 pb, v3 n, float dist, v3 t1, v3 t2,
+                         long long loc) {
+  const size_t NS = (size_t)N * SB_MAXCONTACT, s = (size_t)e * SB_MAXCONTACT + i;
+  crep[CREP_COL_A * NS + s] = __int_as_float(ca);
+  crep[CREP_COL_B * NS + s] = __int_as_float(cb);
+  st3(crep + CREP_POS_A * NS + 3 * s, pa);
+  st3(crep + CREP_POS_B * NS + 3 * s, pb);
+  st3(crep + CREP_NORMAL * NS + 3 * s, n);
+  crep[CREP_DIST * NS + s] = dist;
+  crep[CREP_F1 * NS + s] = __int_as_float((int)(unsigned)(loc & 0xffffffffll));
+  crep[CREP_F2 * NS + s] = __int_as_float((int)(loc >> 32));
+  st3(crep + CREP_DIR1 * NS + 3 * s, t1);
+  st3(crep + CREP_DIR2 * NS + 3 * s, t2);
+}
+
 struct SV {              // one env's column: q i at b[i * stride]
   float4* b;
   int stride;
@@ -316,10 +342,10 @@ PRB_D ContactSides contact_sides(const DevModel& M, const Contact& c) {
   return s;
 }
 
-// constraint rows of the substep -> record stream / heavy buffers
+// constraint rows of the substep -> record stream / heavy buffers (crep: the contact report's geometry and locators too)
 template <int ND, class WM>
 PRB_D void phase_rows_stream(const DevModel& M, WM& W, int lane, int e, int N, const SV& S, float4* __restrict__ hbuf,
-                             int* __restrict__ heavy_cnt) {
+                             int* __restrict__ heavy_cnt, float* __restrict__ crep) {
   const float dt = M.params[P_DT], erp = M.params[P_ERP_JOINT], erp2 = M.params[P_ERP_CONTACT];
   const int nd = M.nd;
   // ---- joint rows, one lane per DoF: limits (lane = arm DoF), motors (lane = arm DoF; lanes 16.. = slide bodies), gear (lane 20).
@@ -564,6 +590,10 @@ PRB_D void phase_rows_stream(const DevModel& M, WM& W, int lane, int e, int N, c
     float rhs[4] = {0.f, 0.f, 0.f, 0.f}, invDs[4] = {0.f, 0.f, 0.f, 0.f}, jsl[4] = {0.f, 0.f, 0.f, 0.f};
     float4* rec = s0 ? &R.q(tC0 + off0) : nullptr;           // slot 0 record
     const int rstride = R.stride;
+    if (crep) {                     // a slot-0 contact always makes its env heavy: its record is in the heavy allocation
+      const long long loc = s0 ? (long long)((rec + (size_t)3 * rstride) - hbuf) << 1 : ((long long)(Q_S12 + region_mine + t) << 1) | 1;
+      crep_geometry(crep, N, e, idx, ca, cb, pa, pb, n, c.dist, t1, t2, loc);
+    }
 #pragma unroll 1
     for (int k = 0; k < 4; k++) {
       v3 dir = k == 0 ? n : (k == 1 ? n : (k == 2 ? t1 : t2));
@@ -660,7 +690,8 @@ __global__ void __launch_bounds__(32 * SetupCfg::WPB, PRB_SETUP_MINB) prb_setup_
                                                                          float* __restrict__ sbuf, DevOut O, int N, int flags,
                                                                          float4* __restrict__ hbuf, int* __restrict__ heavy_cnt,
                                                                          const unsigned char* __restrict__ active,
-                                                                         const int* __restrict__ elist = nullptr, int n_list = 0) {
+                                                                         const int* __restrict__ elist = nullptr, int n_list = 0,
+                                                                         float* __restrict__ crep = nullptr) {
   typedef SetupMemT<SetupCfg> WM;
   PRB_SMEM_DECL2;
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -699,8 +730,9 @@ __global__ void __launch_bounds__(32 * SetupCfg::WPB, PRB_SETUP_MINB) prb_setup_
     if (on) phase_vstar(M, W, lane);
     SETUP_ALIGN();
     if (on) {
-      phase_rows_stream<ND>(M, W, lane, e, N, S, hbuf, heavy_cnt);
+      phase_rows_stream<ND>(M, W, lane, e, N, S, hbuf, heavy_cnt, crep);
       __syncwarp();
+      if (crep && lane == 0) crep_count(crep, N)[e] = W.n_contact;
       // a dropped contact marks the env; the mark is counted (once per env step) by the launch that observes
       if (lane == 0 && W.overflow) { if (O.ovf_env) O.ovf_env[e] = 1; else if (O.overflow) atomicAdd(O.overflow, 1ull); }
       if (lane == 0 && O.dbg) { O.dbg[4 * e] = W.dbg_u | (W.dbg_a << 8); O.dbg[4 * e + 1] = W.dbg_c; O.dbg[4 * e + 2] = W.dbg_p; O.dbg[4 * e + 3] = W.n_jrow | (W.overflow << 8); }
@@ -1147,7 +1179,10 @@ PRB_D void free_sweeps(BV& V, float4* sl, float4* Gr, bool live, int nc, int ns,
 
 __global__ void __launch_bounds__(PGS_BLOCK) prb_pgs_free_kernel(const DevModel* __restrict__ Mp, float* __restrict__ sbuf, int N,
                                                                 const unsigned char* __restrict__ active,
-                                                                const int* __restrict__ elist = nullptr, int n_list = 0) {
+                                                                const int* __restrict__ elist = nullptr, int n_list = 0,
+                                                                int writeback = 0) {
+  // writeback: the staged records (with their impulses) are copied back to the stream after the sweeps, for the contact
+  // report.  Records beyond the stage were updated in place; the stage never holds part of one.
   PRB_PGS_SMEM_DECL;
   const int lane = threadIdx.x;
   const int slot = blockIdx.y + 1;
@@ -1212,6 +1247,8 @@ __global__ void __launch_bounds__(PGS_BLOCK) prb_pgs_free_kernel(const DevModel*
 #pragma unroll
           for (int k = 0; k < 6; k++) gd[((o + k) >> 2) * 128 + ((o + k) & 3)] = v6[k];
         }
+      if (writeback)
+        for (int q = 0; q < min(t_spin + ns, PGS_STAGE_F); q++) Gr[q * 32] = sl[q * 32];
     }
     __syncwarp();
   }
@@ -1379,7 +1416,10 @@ PRB_D void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::
 // be read in place beyond the stage)
 template <int ND, bool INPLACE, int LANES>
 __global__ void __launch_bounds__(32) prb_pgs_arm_kernel(const DevModel* __restrict__ Mp, float* __restrict__ sbuf, float4* __restrict__ hcls,
-                                                                int* __restrict__ heavy_cnt, int capq, int bufq) {
+                                                                int* __restrict__ heavy_cnt, int capq, int bufq, int writeback = 0) {
+  // writeback: after the sweeps the impulse quad (+3) of every staged contact record is copied back to the class buffer, for
+  // the contact report.  Only staged records: INPLACE records read beyond the stage were updated there, and the stage's
+  // stale copy of their first q must not overwrite them.
   constexpr int lanes = LANES;
   PRB_PGS_SMEM_DECL;
   const int lane = threadIdx.x;
@@ -1392,6 +1432,7 @@ __global__ void __launch_bounds__(32) prb_pgs_arm_kernel(const DevModel* __restr
   __syncwarp();
   unsigned parity = 0;
 #endif
+  __shared__ int wb_bundle;           // the bundle being solved (read back by the write-back)
   float sminv[PRB_MAXSLIDE];
 #pragma unroll
   for (int s = 0; s < PRB_MAXSLIDE; s++) sminv[s] = s < M.n_slide ? M.slide_minv[s] : 0.f;
@@ -1401,6 +1442,7 @@ __global__ void __launch_bounds__(32) prb_pgs_arm_kernel(const DevModel* __restr
     if (lane == 0) b = atomicAdd(heavy_cnt + 2, 1);
     b = __shfl_sync(FULL, b, 0);
     if (b >= nb) break;
+    if (writeback && lane == 0) wb_bundle = b;
     float4* Gb = hcls + (size_t)b * ((size_t)bufq * lanes);
     // ---- stage the bundle: capq x lanes float4, contiguous in the class buffer
 #ifndef PRB_EMU
@@ -1472,6 +1514,20 @@ __global__ void __launch_bounds__(32) prb_pgs_arm_kernel(const DevModel* __restr
     }
 #undef ARM_REC
     if (valid) island_store(M, V, sbuf, e, info, true);
+    if (writeback && valid) {
+      // the bundle's global column and its records' start are derived again from shared memory: no value of the staging
+      // stays live across the sweeps, which keep their registers
+      float4* gw = hcls + (size_t)wb_bundle * ((size_t)bufq * lanes) + lane;
+      const float4* sw = sm + lane;
+      const int hw = __float_as_int(sw[R0_HQ * lanes].y), njw = hw & 0xff, ncw = (hw >> 8) & 0xff;
+      int t = R0_JROW + njw + ((njw + 3) >> 2);
+      for (int k = 0; k < ncw; k++) {
+        const bool staged = !(INPLACE && t + CR_MAX_Q > capq);
+        const float4* r = (staged ? sw : gw) + (size_t)t * lanes;
+        if (staged) gw[(size_t)(t + 3) * lanes] = r[3 * lanes];
+        t += __float_as_int(r[0].x) >> 16;
+      }
+    }
     __syncwarp();                                          // the stage is re-filled by the next bundle
   }
 }

@@ -18,6 +18,9 @@ library's buffers).
 With record_images=True every observation also carries 'img' (environments.py:841-845): a uint8 [N,H,W,3] frame of
 `camera` (default: camera.default_camera) rendered on the GPU by prb_render after the step.  render() / render_device()
 draw any other camera (e.g. camera.gripper_camera) with optional depth and segmentation.
+
+With record_contacts=True every step also fills the contact report (PyBullet's getContactPoints after stepSimulation, for
+all envs at once): contacts_device() / contacts() return each env's contact points and forces of the step's last substep.
 """
 import ctypes
 
@@ -35,8 +38,8 @@ OBS_KEYS = OUT_KEYS[:9]
 class _DevArray:
     """Exposes a library-owned device buffer through __cuda_array_interface__ (zero-copy)."""
 
-    def __init__(self, ptr, shape, owner):
-        self.__cuda_array_interface__ = {'shape': tuple(shape), 'typestr': '<f4', 'data': (int(ptr), False),
+    def __init__(self, ptr, shape, owner, typestr='<f4'):
+        self.__cuda_array_interface__ = {'shape': tuple(shape), 'typestr': typestr, 'data': (int(ptr), False),
                                          'version': 2, 'strides': None}
         self._owner = owner
 
@@ -45,7 +48,7 @@ class VecPlayEnv:
     env_id = None
 
     def __init__(self, env_id=None, num_envs=1, device=0, seed=1234, env_offset=0, sparse=True, model=None,
-                 record_images=False, camera=None):
+                 record_images=False, camera=None, record_contacts=False):
         import torch  # device memory / streams only
         self.torch = torch
         env_id = env_id or self.env_id
@@ -110,6 +113,22 @@ class VecPlayEnv:
         self._img = None
         if self.record_images:
             self._img = torch.empty((N, self.camera.height, self.camera.width, 3), dtype=torch.uint8, device=self.device)
+        # contact report: allocated by the library when first enabled
+        self._record_contacts = False
+        self._contact_views = None
+        self.record_contacts = record_contacts
+
+    @property
+    def record_contacts(self):
+        """True: every step / substeps call refreshes the contact report (contacts_device, contacts)."""
+        return self._record_contacts
+
+    @record_contacts.setter
+    def record_contacts(self, on):
+        on = bool(on)
+        if on != self._record_contacts:
+            _lib.check(self.L, self._h, self.L.prb_enable_contacts(self._h, 1 if on else 0))
+            self._record_contacts = on
 
     # ------------------------------------------------------------------ helpers
     def _stream(self):
@@ -309,6 +328,42 @@ class VecPlayEnv:
     def render_box_tests(self):
         """Pixel-box tests the renders of this handle have run (after tile culling)."""
         return int(self.L.prb_render_box_tests(self._h))
+
+    # ------------------------------------------------------------------ contact report
+    def contacts_device(self):
+        """The contacts of the last physics substep of the most recent step (include/prb.h, prb_contacts): dict of CUDA
+        tensors 'count' int32 [N]; 'collider_a', 'collider_b' int32 [N,64] (model collider indices, the ids of
+        render(segmentation=True)); 'position_on_a', 'position_on_b', 'normal_on_b' float32 [N,64,3] (world, m; the normal
+        points from B to A); 'distance', 'normal_force', 'lateral_friction_1', 'lateral_friction_2' float32 [N,64] (m; N);
+        'lateral_friction_dir_1', 'lateral_friction_dir_2' float32 [N,64,3]; and 'body_a', 'body_b' (-1 static, 0 arm,
+        1.. free bodies, then slide bodies), 'link_a', 'link_b' (PyBullet link index) int32 [N,64] looked up from the
+        collider ids.  Entries past count hold -1 (ids) and 0 (floats).  All but the four looked-up arrays are zero-copy
+        views of the library's buffers, overwritten by the next step."""
+        t = self.torch
+        if self._contact_views is None:
+            c = _lib.PrbContacts()
+            _lib.check(self.L, self._h, self.L.prb_get_contacts(self._h, ctypes.byref(c)))
+            N, K = self.num_envs, int(c.max_contacts)
+            with t.cuda.device(self.device):
+                v = {'count': t.as_tensor(_DevArray(c.count, (N,), self, '<i4'), device=self.device)}
+                for name, ty, k in _lib.CONTACT_FIELDS:
+                    shape = (N, K) if k == 1 else (N, K, k)
+                    v[name] = t.as_tensor(_DevArray(getattr(c, name), shape, self, '<' + ty), device=self.device)
+            n_col = int(self.model['n_col'])
+            tables = {key: t.as_tensor(np.asarray(self.model[key])[:n_col].astype(np.int32), device=self.device)
+                      for key in ('col_body', 'col_urdf_link')}
+            self._contact_views = (v, tables)
+        v, tables = self._contact_views
+        d = dict(v)
+        for side in ('a', 'b'):
+            ids = v['collider_' + side]
+            for out, key in (('body_', 'col_body'), ('link_', 'col_urdf_link')):
+                d[out + side] = t.where(ids >= 0, tables[key][ids.clamp(min=0).long()], ids)
+        return d
+
+    def contacts(self):
+        """contacts_device() as numpy arrays."""
+        return {k: v.cpu().numpy() for k, v in self.contacts_device().items()}
 
     # ------------------------------------------------------------------ raw state (tests, checkpoints)
     def get_state(self):
