@@ -197,6 +197,41 @@ int prb_enable_contacts(prb_handle* h, int32_t enable);
 /* Device pointers of the report (handle-owned; valid until prb_destroy).  Fails if the report was never enabled. */
 int prb_get_contacts(prb_handle* h, prb_contacts* out);
 
+/* Per-env dynamics, like PyBullet's changeDynamics() on each client: every env gets its own collider friction and
+ * free-body mass, inertia and damping.  Off by default: every env runs with the model's values and nothing is allocated.
+ * prb_enable_dynamics(h, 1) allocates the table (the first time) and, on every off -> on, fills every env's row with the
+ * model's values; prb_enable_dynamics(h, 0) returns to the model's values and keeps the table.  With PRB_PIPELINE=fused
+ * enabling fails (PRB_ERR_INVALID).  The table is not part of the state row (prb_get_state / prb_set_state).
+ *
+ * The arrays are handle-owned device memory (valid until prb_destroy); callers may write them directly.  A write takes
+ * effect from the next physics substep issued on the same stream.  Values must be finite, mass and inertia > 0, friction
+ * and damping >= 0.  The friction of a contact is the product of its colliders' lateral frictions, clamped to +-10; its
+ * torsional coefficient is spinning_friction * lateral_friction summed over its two colliders. */
+typedef struct prb_dynamics {
+  float* lateral_friction;        /* [N, n_col]      per collider (the model's col_friction) */
+  float* spinning_friction;       /* [N, n_col]      per collider (the model's col_spin) */
+  float* mass;                    /* [N, n_free]     kg, free bodies */
+  float* local_inertia_diagonal;  /* [N, n_free, 3]  kg m^2, principal moments about the COM */
+  float* linear_damping;          /* [N, n_free] */
+  float* angular_damping;         /* [N, n_free] */
+  int32_t num_envs, n_col, n_free;
+} prb_dynamics;
+int prb_enable_dynamics(prb_handle* h, int32_t enable);
+/* Device pointers of the table.  Fails if the table was never enabled. */
+int prb_get_dynamics(prb_handle* h, prb_dynamics* out);
+
+/* [lo, hi] scale of the model's value; lo = hi = 1 keeps the model's value exactly. */
+typedef struct prb_dynamics_ranges {
+  float lateral_friction[2], spinning_friction[2];        /* one draw per body (static scene, arm, each free / slide body) */
+  float mass[2], linear_damping[2], angular_damping[2];   /* one draw per free body; the inertia diagonal follows mass */
+} prb_dynamics_ranges;
+/* Draws new dynamics for the envs of mask_dev (uint8 [N] on the device; NULL: every env): value = model value * s,
+ * s ~ U[lo, hi], in fp32, never compounding earlier draws.  The draws depend only on the seed, the global env id
+ * (env_offset + e) and the env's reset counter, so calling this before prb_reset gives each episode its own dynamics
+ * (prb_reset does not draw on its own; the objects then settle with their new mass).  Fails (PRB_ERR_INVALID, before any
+ * launch) unless the table is enabled and every bound is finite with 0 <= lo <= hi, and 0 < lo for mass. */
+int prb_randomize_dynamics(prb_handle* h, const prb_dynamics_ranges* r, const uint8_t* mask_dev, void* stream);
+
 /* Number of kernels launched by this handle since creation (bench.py reports it). */
 int64_t prb_launch_count(prb_handle* h);
 /* Env steps (since creation; a reset counts as one) in which a contact had to be dropped because the per-env

@@ -15,6 +15,7 @@
 #include "prb_reset.cuh"
 #include "prb_render.cuh"
 #include "prb_contacts.cuh"
+#include "prb_dynamics.cuh"
 
 struct prb_handle {
   DevModel hm;
@@ -61,6 +62,8 @@ struct prb_handle {
   unsigned long long* render_tests = nullptr;   // pixel-box tests of prb_render (allocated by the first render)
   float* crep = nullptr;           // contact report (prb_stream.cuh layout; allocated when first enabled)
   int contacts = 0;                // 1: prb_step / prb_substeps refresh the contact report
+  float* dyn = nullptr;            // per-env dynamics table (prb_stream.cuh layout; allocated when first enabled)
+  int dynamics = 0;                // 1: every setup launch reads the table instead of the model
   std::string err;
 };
 
@@ -93,6 +96,8 @@ struct DevGuard {
 // With the contact report enabled, a step of all envs (not a reset's masked settle steps) also fills the report from
 // its last substep: that substep's setup launch writes the contacts, its solvers write their impulses back, and one
 // prb_contact_report_kernel launch after the final setup launch writes the forces.
+// With the per-env dynamics table enabled, every setup launch (masked and listed ones too, so that a reset's settle
+// substeps run with the env's own masses and frictions) reads it.
 template <int ND>
 static int launch_step(prb_handle* h, int nsub, int observe, cudaStream_t s, const unsigned char* active = nullptr,
                        const int* elist = nullptr, int n_list = 0) {
@@ -128,7 +133,7 @@ static int launch_step(prb_handle* h, int nsub, int observe, cudaStream_t s, con
     if (timed && h->n_evk < 62) CK(h, cudaEventRecord(h->evk[h->n_evk++], s));
     if (i < nsub) CK(h, cudaMemsetAsync(h->heavy_cnt, 0, 4 * ARM_NCLASS * sizeof(int), s));
     prb_setup_kernel<ND><<<gs, bs, h->smem, s>>>(h->dm, h->state, h->sbuf, h->O, N, flags, h->hbuf, h->heavy_cnt, active, elist, n_list,
-                                                    wb ? h->crep : nullptr);
+                                                    wb ? h->crep : nullptr, h->dynamics ? h->dyn : nullptr);
     h->launches++;
     if (i < nsub) {
       if (timed && h->n_evk < 62) CK(h, cudaEventRecord(h->evk[h->n_evk++], s));
@@ -372,6 +377,7 @@ int prb_destroy(prb_handle* h) {
   cudaFree(h->hbuf); cudaFree(h->heavy_cnt);
   if (h->render_tests) cudaFree(h->render_tests);
   if (h->crep) cudaFree(h->crep);
+  if (h->dyn) cudaFree(h->dyn);
   for (int i = 0; i < 3; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   if (h->ev[0]) for (int i = 0; i < 64; i++) cudaEventDestroy(h->evk[i]);
   }
@@ -655,6 +661,72 @@ int prb_get_contacts(prb_handle* h, prb_contacts* out) {
   out->num_envs = h->N;
   out->max_contacts = SB_MAXCONTACT;
   return PRB_OK;
+}
+
+static bool range_ok(const float* r) {   // finite 0 <= lo <= hi
+  return isfinite(r[0]) && isfinite(r[1]) && r[0] >= 0.f && r[0] <= r[1];
+}
+
+// draws (and, from enable, the model's values: every range (1, 1)) for the envs of mask_dev
+static int draw_dynamics(prb_handle* h, const DynRanges& r, const uint8_t* mask_dev, cudaStream_t s) {
+  prb_randomize_dynamics_kernel<<<(h->N + 127) / 128, 128, 0, s>>>(h->dm, h->state, h->dyn, mask_dev, h->N, h->seed, h->env_offset, r);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  return PRB_OK;
+}
+
+int prb_enable_dynamics(prb_handle* h, int32_t enable) {
+  if (!h) return PRB_ERR_INVALID;
+  if (enable && h->fused) {
+    h->err = "prb_enable_dynamics: PRB_PIPELINE=fused reads the model's dynamics only";
+    return PRB_ERR_INVALID;
+  }
+  DevGuard guard(h->device);
+  if (enable && !h->dynamics) {                    // off -> on: every env starts from the model's values
+    const DevModel& M = h->hm;
+    if (!h->dyn) CK(h, cudaMalloc(&h->dyn, dyn_words(h->N, M.n_col, M.n_free) * sizeof(float)));
+    CK(h, cudaDeviceSynchronize());
+    const DynRanges unit = {{1.f, 1.f}, {1.f, 1.f}, {1.f, 1.f}, {1.f, 1.f}, {1.f, 1.f}};
+    const int rc = draw_dynamics(h, unit, nullptr, nullptr);
+    if (rc != PRB_OK) return rc;
+    CK(h, cudaDeviceSynchronize());
+  }
+  h->dynamics = enable ? 1 : 0;
+  return PRB_OK;
+}
+
+int prb_get_dynamics(prb_handle* h, prb_dynamics* out) {
+  if (!h || !out) return PRB_ERR_INVALID;
+  if (!h->dyn) { h->err = "prb_get_dynamics: the dynamics table was never enabled (prb_enable_dynamics)"; return PRB_ERR_INVALID; }
+  const DevModel& M = h->hm;
+  const int64_t N = h->N;
+  out->lateral_friction = h->dyn + dyn_offset(N, M.n_col, M.n_free, DYN_FRIC);
+  out->spinning_friction = h->dyn + dyn_offset(N, M.n_col, M.n_free, DYN_SPIN);
+  out->mass = h->dyn + dyn_offset(N, M.n_col, M.n_free, DYN_MASS);
+  out->local_inertia_diagonal = h->dyn + dyn_offset(N, M.n_col, M.n_free, DYN_INERTIA);
+  out->linear_damping = h->dyn + dyn_offset(N, M.n_col, M.n_free, DYN_LD);
+  out->angular_damping = h->dyn + dyn_offset(N, M.n_col, M.n_free, DYN_AD);
+  out->num_envs = h->N;
+  out->n_col = M.n_col;
+  out->n_free = M.n_free;
+  return PRB_OK;
+}
+
+int prb_randomize_dynamics(prb_handle* h, const prb_dynamics_ranges* r, const uint8_t* mask_dev, void* stream) {
+  if (!h || !r) return PRB_ERR_INVALID;
+  if (!h->dynamics) { h->err = "prb_randomize_dynamics: the dynamics table is not enabled (prb_enable_dynamics)"; return PRB_ERR_INVALID; }
+  if (!range_ok(r->lateral_friction) || !range_ok(r->spinning_friction) || !range_ok(r->linear_damping) ||
+      !range_ok(r->angular_damping) || !range_ok(r->mass) || !(r->mass[0] > 0.f)) {
+    h->err = "prb_randomize_dynamics: every range needs finite 0 <= lo <= hi (mass: 0 < lo)";
+    return PRB_ERR_INVALID;
+  }
+  DevGuard guard(h->device);
+  DynRanges d;
+  for (int k = 0; k < 2; k++) {
+    d.lateral_friction[k] = r->lateral_friction[k]; d.spinning_friction[k] = r->spinning_friction[k]; d.mass[k] = r->mass[k];
+    d.linear_damping[k] = r->linear_damping[k]; d.angular_damping[k] = r->angular_damping[k];
+  }
+  return draw_dynamics(h, d, mask_dev, (cudaStream_t)stream);
 }
 
 int64_t prb_launch_count(prb_handle* h) { return h ? h->launches : 0; }

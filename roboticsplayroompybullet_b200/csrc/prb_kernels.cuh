@@ -388,12 +388,16 @@ PRB_D void store_state(const DevModel& M, const WM& W, float* st, int lane) {
   }
 }
 
+// Free-body constants of one env, fd[FD_N * b + FD_*] (the split pipeline's setup kernel stages them per env; phase_fk
+// and phase_vstar read the model's own when fd is NULL)
+enum { FD_MASS = 0, FD_INERTIA = 1, FD_LD = 4, FD_AD = 5, FD_N = 6 };
+
 // ============================================================================ kinematics + bias (lane = arm link)
 // Each lane walks its own root->link path, accumulating the frame, the velocity and the
 // velocity-product acceleration (recursive Newton-Euler forward pass with qdd = 0 and gravity
 // folded in as base acceleration); no inter-lane communication.
 template <class WM>
-PRB_D void phase_fk(const DevModel& M, WM& W, int lane, bool dynamics) {
+PRB_D void phase_fk(const DevModel& M, WM& W, int lane, bool dynamics, const float* fd = nullptr) {
   if (lane < M.nd) {
     m3 R = ldm(M.base_rot);
     v3 p = ld3(M.base_pos);
@@ -442,7 +446,8 @@ PRB_D void phase_fk(const DevModel& M, WM& W, int lane, bool dynamics) {
   if (b >= 0 && b < M.n_free) {
     m3 R; quat_to_mat(W.fquat[b], R); stm(W.fR[b], R);
     if (dynamics) {
-      float Dg[6] = {1.0f / M.free_inertia[b][0], 0, 0, 1.0f / M.free_inertia[b][1], 0, 1.0f / M.free_inertia[b][2]}, o[6];
+      const float* I = fd ? fd + FD_N * b + FD_INERTIA : M.free_inertia[b];
+      float Dg[6] = {1.0f / I[0], 0, 0, 1.0f / I[1], 0, 1.0f / I[2]}, o[6];
       rot_sym(R, Dg, o);
       for (int k = 0; k < 6; k++) W.fIinv[b][k] = o[k];
     }
@@ -548,18 +553,18 @@ PRB_D void phase_minv(WM& W, int lane) {
 
 // unconstrained velocity update v* = v + dt * a  (lane = velocity DoF); result in W.vs and returned
 template <class WM>
-PRB_D float phase_vstar(const DevModel& M, WM& W, int lane) {
+PRB_D float phase_vstar(const DevModel& M, WM& W, int lane, const float* fd = nullptr) {
   const float dt = M.params[P_DT], g = M.params[P_GRAVITY_Z], vmax = M.params[P_MAX_COORD_VEL];
   const int nd = M.nd;
   // free bodies: one lane per body does the coupled 3-vector algebra
   int b = lane - nd;
   if (b >= 0 && b < M.n_free) {
     m3 R = ldm(W.fR[b]);
-    float kl = M.free_ld[b], ka = M.free_ad[b];
+    float kl = fd ? fd[FD_N * b + FD_LD] : M.free_ld[b], ka = fd ? fd[FD_N * b + FD_AD] : M.free_ad[b];
     v3 vl = ld3(W.fvel[b]), w = ld3(W.fang[b]);
     v3 acc = V3(0, 0, g) + vl * (-(kl + kl * norm(vl)));
     v3 wb = tmul(R, w);
-    v3 Id = ld3(M.free_inertia[b]);
+    v3 Id = ld3(fd ? fd + FD_N * b + FD_INERTIA : M.free_inertia[b]);
     v3 gy = cross(wb, V3(Id.x * wb.x, Id.y * wb.y, Id.z * wb.z));
     v3 wdb = V3(-gy.x / Id.x, -gy.y / Id.y, -gy.z / Id.z) + wb * (-(ka + ka * norm(wb)));
     v3 wd = mul(R, wdb);

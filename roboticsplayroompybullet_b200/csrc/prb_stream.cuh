@@ -163,6 +163,16 @@ PRB_D void crep_geometry(float* crep, int N, int e, int i, int ca, int cb, v3 pa
   st3(crep + CREP_DIR2 * NS + 3 * s, t2);
 }
 
+// ---- per-env dynamics table (prb_enable_dynamics, include/prb.h): one allocation, one dense fp32 array per field in the
+// order of prb_dynamics: lateral_friction [N, n_col], spinning_friction [N, n_col], mass [N, n_free],
+// local_inertia_diagonal [N, n_free, 3], linear_damping [N, n_free], angular_damping [N, n_free].
+enum { DYN_FRIC = 0, DYN_SPIN, DYN_MASS, DYN_INERTIA, DYN_LD, DYN_AD };
+PRB_HD size_t dyn_offset(int64_t N, int n_col, int n_free, int f) {
+  const size_t c = (size_t)N * n_col, b = (size_t)N * n_free;
+  return f <= DYN_SPIN ? f * c : 2 * c + (f == DYN_MASS ? 0 : (f == DYN_INERTIA ? b : (f == DYN_LD ? 4 * b : 5 * b)));
+}
+PRB_HD size_t dyn_words(int64_t N, int n_col, int n_free) { return dyn_offset(N, n_col, n_free, DYN_AD) + (size_t)N * n_free; }
+
 struct SV {              // one env's column: q i at b[i * stride]
   float4* b;
   int stride;
@@ -228,6 +238,9 @@ struct SetupMemT {
   float sp[PRB_MAXSLIDE][3], sR[PRB_MAXSLIDE][9];
   float Minv[PRB_MAXD][PRB_MAXD + 1], Q[PRB_MAXD];
   float vs[32];
+  float fdyn[PRB_MAXFREE * FD_N];                 // the env's free-body constants (phase_fk FD_* layout)
+  const float* fric;                              // the env's collider friction row: the dynamics table's or the model's
+  const float* spin;
   unsigned short ovl[CFG::MAXOVL];
   int n_ovl, n_contact, n_jrow, pool_used, overflow;
   int dbg_a, dbg_c, dbg_p, dbg_u;
@@ -294,7 +307,7 @@ PRB_D float side_row(const DevModel& M, const WM& W, int col, v3 pt, v3 dir, flo
     const int b = body - 1, o = M.nd + 6 * b;
     v3 t = angular ? dir : cross(pt - ld3(W.fpos[b]), dir);
     v3 jl = angular ? V3(0, 0, 0) : dir * sign, ja = t * sign;
-    float im = 1.0f / M.free_mass[b];
+    float im = 1.0f / W.fdyn[FD_N * b + FD_MASS];
     v3 bl = jl * im, ba = symmul(W.fIinv[b], ja);
     float J[6] = {jl.x, jl.y, jl.z, ja.x, ja.y, ja.z}, B[6] = {bl.x, bl.y, bl.z, ba.x, ba.y, ba.z};
     float r = 0.f;
@@ -328,7 +341,8 @@ PRB_D float4 jrow_q(const DevModel& M, int d, int d2, int neg, int sym, float rh
 // the two sides of a contact ordered by kind (P = the higher-ranked side: arm > slide > free > static), their groups
 // (0: arm + slide bodies, 1 + b: free body b, -1: static) and the torsional friction coefficient
 struct ContactSides { int colP, colS, kP, kS, grpP, grpS; bool swapped, has_spin; float spin; };
-PRB_D ContactSides contact_sides(const DevModel& M, const Contact& c) {
+template <class WM>
+PRB_D ContactSides contact_sides(const DevModel& M, const WM& W, const Contact& c) {
   ContactSides s;
   const int ca = c.cols & 0xff, cb = (c.cols >> 8) & 0xff;
   const int kA = body_kind(M, col_dyn_body(M, ca)), kB = body_kind(M, col_dyn_body(M, cb));
@@ -337,7 +351,7 @@ PRB_D ContactSides contact_sides(const DevModel& M, const Contact& c) {
   s.kP = s.swapped ? kB : kA; s.kS = s.swapped ? kA : kB;
   s.grpP = s.kP == K_FREE ? M.col_body[s.colP] : 0;
   s.grpS = s.kS == K_STATIC ? -1 : (s.kS == K_FREE ? M.col_body[s.colS] : 0);
-  s.spin = M.col_spin[ca] * M.col_fric[ca] + M.col_spin[cb] * M.col_fric[cb];
+  s.spin = __ldg(W.spin + ca) * __ldg(W.fric + ca) + __ldg(W.spin + cb) * __ldg(W.fric + cb);
   s.has_spin = s.spin > 0.f;
   return s;
 }
@@ -415,7 +429,7 @@ PRB_D void phase_rows_stream(const DevModel& M, WM& W, int lane, int e, int N, c
         int lo_ = 0, hi_ = 0;
         bool two = false;
         if (idx < nc) {
-          const ContactSides cs = contact_sides(M, W.ct[idx]);
+          const ContactSides cs = contact_sides(M, W, W.ct[idx]);
           two = cs.grpS >= 0 && cs.grpS != cs.grpP;
           lo_ = min(cs.grpP, cs.grpS); hi_ = max(cs.grpP, cs.grpS);
         }
@@ -437,7 +451,7 @@ PRB_D void phase_rows_stream(const DevModel& M, WM& W, int lane, int e, int N, c
     if (h < nh) {
       const int idx = h * 32 + lane;
       if (idx < nc) {
-        const ContactSides cs = contact_sides(M, W.ct[idx]);
+        const ContactSides cs = contact_sides(M, W, W.ct[idx]);
         slot_[h] = cs.grpP == 0 ? 0 : slotf[cs.grpP - 1];
         spin_[h] = cs.has_spin;
         if (slot_[h] == 0) size0_[h] = CR_BASE_Q + (cs.kP == K_ARM ? (cs.has_spin ? 24 : 18) : 0);
@@ -537,7 +551,7 @@ PRB_D void phase_rows_stream(const DevModel& M, WM& W, int lane, int e, int N, c
     float4 i0 = make_float4(0.f, 0.f, 0.f, 0.f), i1 = i0;
     if (b < M.n_free) {
       i0 = make_float4(W.fIinv[b][0], W.fIinv[b][1], W.fIinv[b][2], W.fIinv[b][3]);
-      i1 = make_float4(W.fIinv[b][4], W.fIinv[b][5], 1.0f / M.free_mass[b], 0.f);
+      i1 = make_float4(W.fIinv[b][4], W.fIinv[b][5], 1.0f / W.fdyn[FD_N * b + FD_MASS], 0.f);
     }
     R.q(R0_BODY + 2 * b) = i0; R.q(R0_BODY + 2 * b + 1) = i1;
     if (heavy) { S.q(Q_ST + R0_BODY + 2 * b) = i0; S.q(Q_ST + R0_BODY + 2 * b + 1) = i1; }    // the free-body kernel reads the stream
@@ -560,7 +574,7 @@ PRB_D void phase_rows_stream(const DevModel& M, WM& W, int lane, int e, int N, c
     const int idx = h * 32 + lane;
     if (idx >= nc) continue;
     const Contact c = W.ct[idx];
-    const ContactSides cs = contact_sides(M, c);
+    const ContactSides cs = contact_sides(M, W, c);
     const int colP = cs.colP, colS = cs.colS, kP = cs.kP, kS = cs.kS;
     const bool swapped = cs.swapped, has_spin = cs.has_spin;
     const float spin = cs.spin;
@@ -583,7 +597,7 @@ PRB_D void phase_rows_stream(const DevModel& M, WM& W, int lane, int e, int N, c
       cfm = 1.0f / denom; er = dt * kk / denom;
     }
     cfm /= dt;
-    const float mu = clampf(M.col_fric[ca] * M.col_fric[cb], -10.f, 10.f);
+    const float mu = clampf(__ldg(W.fric + ca) * __ldg(W.fric + cb), -10.f, 10.f);
     v3 t1, t2;
     plane_space(n, t1, t2);
     float cfms = 0.f;
@@ -682,6 +696,29 @@ PRB_D int env_of(int i, int N, const unsigned char* active, const int* elist, in
   return i;
 }
 
+// The env's dynamics constants for this launch: its row of the per-env table (dyn, prb_enable_dynamics), else the model's.
+// Free-body constants are copied into W.fdyn; the friction rows are read in place through W.fric / W.spin (L1-resident,
+// a few reads per contact).
+template <class WM>
+PRB_D void stage_dynamics(const DevModel& M, WM& W, int lane, int e, int N, const float* __restrict__ dyn) {
+  const int nc = M.n_col, nf = M.n_free;
+  if (lane < FD_N * nf) {
+    const int b = lane / FD_N, k = lane - FD_N * b;
+    float v;
+    if (dyn) {
+      const size_t f = dyn_offset(N, nc, nf, k == FD_MASS ? DYN_MASS : (k < FD_LD ? DYN_INERTIA : (k == FD_LD ? DYN_LD : DYN_AD)));
+      v = dyn[f + (k < FD_LD && k != FD_MASS ? (size_t)3 * (e * nf + b) + (k - FD_INERTIA) : (size_t)e * nf + b)];
+    } else {
+      v = k == FD_MASS ? M.free_mass[b] : (k < FD_LD ? M.free_inertia[b][k - FD_INERTIA] : (k == FD_LD ? M.free_ld[b] : M.free_ad[b]));
+    }
+    W.fdyn[lane] = v;
+  }
+  if (lane == 0) {
+    W.fric = dyn ? dyn + dyn_offset(N, nc, nf, DYN_FRIC) + (size_t)e * nc : M.col_fric;
+    W.spin = dyn ? dyn + dyn_offset(N, nc, nf, DYN_SPIN) + (size_t)e * nc : M.col_spin;
+  }
+}
+
 #ifndef PRB_SETUP_MINB
 #define PRB_SETUP_MINB 2       // 2 x 8 warps per SM = 128 registers per thread; measured r2l: 1 block (natural register count) 43.9 ms of setup per env step, 2 x 10 warps at 96 registers (spills) 40.2 ms, this 31.8 ms
 #endif
@@ -691,7 +728,8 @@ __global__ void __launch_bounds__(32 * SetupCfg::WPB, PRB_SETUP_MINB) prb_setup_
                                                                          float4* __restrict__ hbuf, int* __restrict__ heavy_cnt,
                                                                          const unsigned char* __restrict__ active,
                                                                          const int* __restrict__ elist = nullptr, int n_list = 0,
-                                                                         float* __restrict__ crep = nullptr) {
+                                                                         float* __restrict__ crep = nullptr,
+                                                                         const float* __restrict__ dyn = nullptr) {
   typedef SetupMemT<SetupCfg> WM;
   PRB_SMEM_DECL2;
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -708,6 +746,7 @@ __global__ void __launch_bounds__(32 * SetupCfg::WPB, PRB_SETUP_MINB) prb_setup_
   if (on) {
     load_state(M, W, st, lane);
     if (lane == 0) { W.overflow = 0; W.dbg_a = 0; W.dbg_c = 0; W.dbg_p = 0; W.dbg_u = 0; }
+    stage_dynamics(M, W, lane, e, N, dyn);
     __syncwarp();
     if (flags & SETUP_INTEGRATE) {
       float vstar = 0.f, dv = 0.f;
@@ -717,7 +756,7 @@ __global__ void __launch_bounds__(32 * SetupCfg::WPB, PRB_SETUP_MINB) prb_setup_
   }
   if (flags & SETUP_BUILD) {
     SETUP_ALIGN();
-    if (on) phase_fk(M, W, lane, true);
+    if (on) phase_fk(M, W, lane, true, W.fdyn);
     SETUP_ALIGN();
     if (on) phase_collide_broad(M, W, lane);
     SETUP_ALIGN();
@@ -727,7 +766,7 @@ __global__ void __launch_bounds__(32 * SetupCfg::WPB, PRB_SETUP_MINB) prb_setup_
     SETUP_ALIGN2();
     if (on) phase_minv<ND>(W, lane);
     SETUP_ALIGN2();
-    if (on) phase_vstar(M, W, lane);
+    if (on) phase_vstar(M, W, lane, W.fdyn);
     SETUP_ALIGN();
     if (on) {
       phase_rows_stream<ND>(M, W, lane, e, N, S, hbuf, heavy_cnt, crep);

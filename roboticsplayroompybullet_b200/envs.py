@@ -21,7 +21,13 @@ draw any other camera (e.g. camera.gripper_camera) with optional depth and segme
 
 With record_contacts=True every step also fills the contact report (PyBullet's getContactPoints after stepSimulation, for
 all envs at once): contacts_device() / contacts() return each env's contact points and forces of the step's last substep.
+
+With per_env_dynamics=True every env has its own collider friction and free-body mass, inertia and damping (PyBullet's
+changeDynamics per client): change_dynamics() sets them, dynamics_device() / dynamics() return them.  With
+randomize_dynamics={field: (lo, hi)} every sampled reset first draws new values for the envs it resets (domain
+randomization).
 """
+import math
 import ctypes
 
 import numpy as np
@@ -48,7 +54,7 @@ class VecPlayEnv:
     env_id = None
 
     def __init__(self, env_id=None, num_envs=1, device=0, seed=1234, env_offset=0, sparse=True, model=None,
-                 record_images=False, camera=None, record_contacts=False):
+                 record_images=False, camera=None, record_contacts=False, per_env_dynamics=False, randomize_dynamics=None):
         import torch  # device memory / streams only
         self.torch = torch
         env_id = env_id or self.env_id
@@ -117,6 +123,45 @@ class VecPlayEnv:
         self._record_contacts = False
         self._contact_views = None
         self.record_contacts = record_contacts
+        # per-env dynamics table: allocated by the library when first enabled
+        self._per_env_dynamics = False
+        self._dyn_views = None
+        self._dyn_ranges = None
+        self.per_env_dynamics = per_env_dynamics
+        self.randomize_dynamics = randomize_dynamics
+
+    @property
+    def per_env_dynamics(self):
+        """True: every env runs with its own row of the dynamics table (dynamics_device, change_dynamics).  Turning it on
+        fills every row with the model's values; turning it off also turns randomize_dynamics off."""
+        return self._per_env_dynamics
+
+    @per_env_dynamics.setter
+    def per_env_dynamics(self, on):
+        on = bool(on)
+        if on != self._per_env_dynamics:
+            _lib.check(self.L, self._h, self.L.prb_enable_dynamics(self._h, 1 if on else 0))
+            self._per_env_dynamics = on
+        if not on:
+            self._dyn_ranges = None
+
+    @property
+    def randomize_dynamics(self):
+        """{field: (lo, hi)} scale ranges of the model's values that every sampled reset draws from (None: no draw).
+        Fields: lateral_friction, spinning_friction (one draw per body), mass, linear_damping, angular_damping (one per
+        free body; the inertia follows mass); the ones not given keep (1, 1).  Setting it turns per_env_dynamics on."""
+        if self._dyn_ranges is None:
+            return None
+        return {k: tuple(getattr(self._dyn_ranges, k)) for k in _lib.DYNAMICS_RANGE_FIELDS}
+
+    @randomize_dynamics.setter
+    def randomize_dynamics(self, spec):
+        if spec is None:
+            self._dyn_ranges = None
+            return
+        r = dynamics_ranges(spec)
+        self.per_env_dynamics = True
+        self._dyn_ranges = r
 
     @property
     def record_contacts(self):
@@ -188,6 +233,8 @@ class VecPlayEnv:
         if mask is not None:
             self._mask = mask.to(self.device, self.torch.uint8).contiguous()
             mp = ctypes.c_void_p(self._mask.data_ptr())
+        if o is None and self._dyn_ranges is not None:      # new dynamics before the objects settle
+            _lib.check(self.L, self._h, self.L.prb_randomize_dynamics(self._h, ctypes.byref(self._dyn_ranges), mp, self._stream()))
         if o is not None:
             ob = o.to(self.device, self.torch.float32).contiguous()
             assert ob.shape == (self.num_envs, self.dims['obs_quat']), 'o must be [num_envs, %d] (obs_quat layout)' % self.dims['obs_quat']
@@ -365,6 +412,62 @@ class VecPlayEnv:
         """contacts_device() as numpy arrays."""
         return {k: v.cpu().numpy() for k, v in self.contacts_device().items()}
 
+    # ------------------------------------------------------------------ per-env dynamics
+    def dynamics_device(self):
+        """The per-env dynamics table (include/prb.h, prb_dynamics) as zero-copy CUDA tensors: 'lateral_friction',
+        'spinning_friction' float32 [N, n_col]; 'mass', 'linear_damping', 'angular_damping' float32 [N, n_free];
+        'local_inertia_diagonal' float32 [N, n_free, 3].  Writes take effect from the next physics substep on the same
+        stream; values must be finite, mass and inertia > 0, friction and damping >= 0."""
+        if self._dyn_views is None:
+            if not self._per_env_dynamics:
+                raise _lib.PrbError('per_env_dynamics is off')
+            d = _lib.PrbDynamics()
+            _lib.check(self.L, self._h, self.L.prb_get_dynamics(self._h, ctypes.byref(d)))
+            N, nc, nf = self.num_envs, int(d.n_col), int(d.n_free)
+            shapes = {'lateral_friction': (N, nc), 'spinning_friction': (N, nc), 'mass': (N, nf),
+                      'local_inertia_diagonal': (N, nf, 3), 'linear_damping': (N, nf), 'angular_damping': (N, nf)}
+            with self.torch.cuda.device(self.device):
+                self._dyn_views = {k: self.torch.as_tensor(_DevArray(getattr(d, k), shapes[k], self), device=self.device)
+                                   for k in _lib.DYNAMICS_FIELDS}
+        return dict(self._dyn_views)
+
+    def dynamics(self):
+        """dynamics_device() as numpy arrays (copies)."""
+        return {k: v.cpu().numpy() for k, v in self.dynamics_device().items()}
+
+    def change_dynamics(self, body, link=-1, mask=None, *, lateral_friction=None, spinning_friction=None, mass=None,
+                        local_inertia_diagonal=None, linear_damping=None, angular_damping=None):
+        """PyBullet's changeDynamics(body, link, ...) for the envs of `mask` (uint8 / bool [N]; None: all).  body: -1 static
+        scene, 0 arm, 1.. free bodies, then slide bodies (the ids of contacts()); link: the PyBullet link index.  A value
+        is a scalar or one per env ([N], [N, 3] for the inertia).  Friction goes to every collider of (body, link); mass,
+        inertia and damping exist for free bodies only.  mass= without local_inertia_diagonal= rescales the inertia by the
+        mass ratio.  Raises ValueError for an unknown (body, link) or a bad value; needs per_env_dynamics."""
+        cols, fb = dynamics_target(self.model, body, link)
+        t, N = self.torch, self.num_envs
+        vals = {'lateral_friction': lateral_friction, 'spinning_friction': spinning_friction, 'mass': mass,
+                'local_inertia_diagonal': local_inertia_diagonal, 'linear_damping': linear_damping,
+                'angular_damping': angular_damping}
+        vals = {k: check_dynamics_value(k, v, N) for k, v in vals.items() if v is not None}
+        if fb is None and any(k not in ('lateral_friction', 'spinning_friction') for k in vals):
+            raise ValueError('mass, inertia and damping belong to free bodies only (body %d is not one)' % body)
+        d = self.dynamics_device()
+        sel = t.ones(N, dtype=t.bool, device=self.device) if mask is None else \
+            t.as_tensor(np.asarray(mask)).to(self.device).reshape(N).bool()
+        dev = lambda v: t.as_tensor(v, dtype=t.float32, device=self.device)
+        for k in ('lateral_friction', 'spinning_friction'):
+            if k in vals:
+                ci = t.as_tensor(cols, dtype=t.long, device=self.device)
+                cur = d[k][:, ci]
+                d[k][:, ci] = t.where(sel[:, None], dev(vals[k])[:, None].expand_as(cur), cur)
+        if 'mass' in vals and 'local_inertia_diagonal' not in vals:
+            ratio = dev(vals['mass']) / d['mass'][:, fb]
+            vals['local_inertia_diagonal'] = (d['local_inertia_diagonal'][:, fb] * ratio[:, None]).cpu().numpy()
+        for k in ('mass', 'local_inertia_diagonal', 'linear_damping', 'angular_damping'):
+            if k in vals:
+                cur = d[k][:, fb]
+                new = dev(vals[k])
+                d[k][:, fb] = t.where(sel[:, None] if cur.dim() == 2 else sel, new, cur)
+
     # ------------------------------------------------------------------ raw state (tests, checkpoints)
     def get_state(self):
         out = np.zeros((self.num_envs, self.buffers.state_dim), np.float32)
@@ -416,6 +519,54 @@ class VecPlayEnv:
         a, b, c = ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int32()
         self.L.prb_kernel_info(self._h, ctypes.byref(a), ctypes.byref(b), ctypes.byref(c))
         return {'smem_bytes_per_block': a.value, 'envs_per_block': b.value, 'regs_per_thread': c.value}
+
+
+def dynamics_ranges(spec):
+    """{field: (lo, hi)} -> prb_dynamics_ranges; fields not given are (1, 1).  ValueError for an unknown field or a bound
+    that is not finite, lo > hi, lo < 0, or a mass lower bound of 0."""
+    r = _lib.PrbDynamicsRanges()
+    for k in _lib.DYNAMICS_RANGE_FIELDS:
+        getattr(r, k)[:] = (1.0, 1.0)
+    for k, v in dict(spec).items():
+        if k not in _lib.DYNAMICS_RANGE_FIELDS:
+            raise ValueError('unknown dynamics range %r (fields: %s)' % (k, ', '.join(_lib.DYNAMICS_RANGE_FIELDS)))
+        lo, hi = (float(x) for x in v)
+        if not (math.isfinite(lo) and math.isfinite(hi) and 0.0 <= lo <= hi) or (k == 'mass' and lo <= 0.0):
+            raise ValueError('%s range (%r, %r): needs finite 0 <= lo <= hi%s' % (k, lo, hi, ', lo > 0' if k == 'mass' else ''))
+        getattr(r, k)[:] = (lo, hi)
+    return r
+
+
+def dynamics_target(model, body, link=-1):
+    """(collider indices of (body, link), free-body index or None) of a compiled model, the ids contacts() reports: body
+    -1 static scene, 0 arm, 1.. free bodies, then slide bodies; link the PyBullet link index.  ValueError if (body, link)
+    has no collider."""
+    nc, nf = int(model['n_col']), int(model['n_free'])
+    cb = np.asarray(model['col_body'])[:nc]
+    cl = np.asarray(model['col_urdf_link'])[:nc]
+    cols = np.nonzero((cb == int(body)) & (cl == int(link)))[0]
+    if len(cols) == 0:
+        raise ValueError('no collider has body %r link %r' % (body, link))
+    return cols, (int(body) - 1 if 1 <= int(body) <= nf else None)
+
+
+def check_dynamics_value(field, v, N):
+    """A change_dynamics value as float32 [N] ([N, 3] for the inertia), broadcast from a scalar (or a 3-vector for the
+    inertia).  ValueError if it is not finite, mass or inertia <= 0, or friction or damping < 0."""
+    a = np.asarray(v, np.float64)
+    shape = (N, 3) if field == 'local_inertia_diagonal' else (N,)
+    try:
+        a = np.broadcast_to(a, shape)
+    except ValueError:
+        raise ValueError('%s: expected a scalar or shape %s, got %s' % (field, shape, a.shape)) from None
+    if not np.isfinite(a).all():
+        raise ValueError('%s: values must be finite' % field)
+    if field in ('mass', 'local_inertia_diagonal'):
+        if not (a > 0).all():
+            raise ValueError('%s: values must be > 0' % field)
+    elif not (a >= 0).all():
+        raise ValueError('%s: values must be >= 0' % field)
+    return np.ascontiguousarray(a, np.float32)
 
 
 # the three registered ids in scope (roboticsPlayroomPybullet/__init__.py:23-26,65-68,91-94)

@@ -45,11 +45,27 @@ class PrbContacts(ctypes.Structure):
                 [('num_envs', ctypes.c_int32), ('max_contacts', ctypes.c_int32)])
 
 
+# prb_dynamics: the per-env dynamics table's device arrays, in struct order
+DYNAMICS_FIELDS = ['lateral_friction', 'spinning_friction', 'mass', 'local_inertia_diagonal', 'linear_damping', 'angular_damping']
+# prb_dynamics_ranges, in struct order
+DYNAMICS_RANGE_FIELDS = ['lateral_friction', 'spinning_friction', 'mass', 'linear_damping', 'angular_damping']
+
+
+class PrbDynamics(ctypes.Structure):
+    _fields_ = ([(n, ctypes.c_void_p) for n in DYNAMICS_FIELDS] +
+                [('num_envs', ctypes.c_int32), ('n_col', ctypes.c_int32), ('n_free', ctypes.c_int32)])
+
+
+class PrbDynamicsRanges(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_float * 2) for n in DYNAMICS_RANGE_FIELDS]
+
+
 # every symbol include/prb.h declares (a CPU test checks the built library exports them all)
 SYMBOLS = ['prb_create', 'prb_destroy', 'prb_reset', 'prb_reset_rounds', 'prb_reset_to', 'prb_set_goal', 'prb_step', 'prb_observe', 'prb_substeps',
            'prb_get_buffers', 'prb_compute_reward', 'prb_get_state', 'prb_set_state', 'prb_step_host',
            'prb_enable_kernel_timing', 'prb_last_kernel_ms', 'prb_last_tier_ms', 'prb_launch_count', 'prb_overflow_count', 'prb_debug_usage', 'prb_kernel_info', 'prb_render', 'prb_render_box_tests',
-           'prb_enable_contacts', 'prb_get_contacts', 'prb_last_error',
+           'prb_enable_contacts', 'prb_get_contacts', 'prb_enable_dynamics', 'prb_get_dynamics', 'prb_randomize_dynamics',
+           'prb_last_error',
            'prb_version']
 
 
@@ -94,6 +110,9 @@ def load():
     L.prb_render_box_tests.restype = i64
     L.prb_enable_contacts.argtypes = [vp, i32]
     L.prb_get_contacts.argtypes = [vp, ctypes.POINTER(PrbContacts)]
+    L.prb_enable_dynamics.argtypes = [vp, i32]
+    L.prb_get_dynamics.argtypes = [vp, ctypes.POINTER(PrbDynamics)]
+    L.prb_randomize_dynamics.argtypes = [vp, ctypes.POINTER(PrbDynamicsRanges), vp, vp]
     L.prb_last_error.argtypes = [vp]
     L.prb_last_error.restype = ctypes.c_char_p
     L.prb_version.restype = ctypes.c_char_p
