@@ -158,6 +158,38 @@ int prb_render(prb_handle* h, const prb_camera* cam, const float* col_rgb_host, 
 /* Pixel-box slab tests prb_render has run since creation (after tile culling; for reports).  Synchronises the device. */
 int64_t prb_render_box_tests(prb_handle* h);
 
+/* Ray casts against the collision boxes of every env, like PyBullet's rayTestBatch() on each client: the nearest hit of
+ * each segment from -> to.  Reads the current state (the state prb_render reads) and writes only the given arrays;
+ * asynchronous on `stream`, no host synchronisation, no allocation, exactly one kernel launch.  Works with either
+ * PRB_PIPELINE.
+ *
+ * Endpoints are given in `frame`: the world (-1) or site s of the arm (the model's site_link[s] / site_pos / site_rot;
+ * 0 is the end effector, the frame of an attached prb_camera, 1 the wrist, 2 and 3 the finger pads), where a point x
+ * is p_s + R_s x in the world.  Results are in the world.  In the box coordinates of collider c the ray is o + t dl,
+ * dl = R_box^T (to - from) (not normalised), t in [0, 1]: an axis with |dl_k| < 1e-12 is parallel and keeps the ray
+ * only if o_k is in [-h_k, h_k]; otherwise t is clipped to the slab.  The box is hit when the clipped t0 <= t1 and
+ * t0 < 1; the nearest hit wins, the lower collider index on equal t0.  (The rule of the step's gripper_proprioception
+ * ray.)  So a ray that starts inside a box hits it at fraction 0, a hit exactly at `to` is a miss, and a zero-length ray
+ * hits only when it starts inside a box.  A ray with a non-finite endpoint is a miss.
+ *
+ * The normal is the world axis of the box slab whose entry set t0, pointing against the ray (the lowest axis on equal
+ * entries); when the ray starts inside the box (no entry > 0) it is -(to - from) / |to - from|, and 0 for a zero-length
+ * ray. */
+typedef struct prb_rays {
+  int32_t num_rays;        /* R per env, 1..16384 */
+  int32_t per_env;         /* 0: from / to are [R,3], shared by every env; 1: [N,R,3] */
+  int32_t frame;           /* -1: world; 0..3: site s of the arm */
+  int32_t reserved;        /* must be 0 */
+  uint64_t collider_mask;  /* bit c set: collider c can be hit (~0: all; bits >= n_col ignored) */
+} prb_rays;
+/* from_dev, to_dev: float device arrays in the layout of r->per_env.  Outputs (device, indexed in 64 bits):
+ * hit_collider_dev int32 [N,R] (required; -1 for a miss), hit_fraction_dev float [N,R] (required; in [0,1), 1 for a
+ * miss), hit_position_dev float [N,R,3] (optional, NULL; world, 0 for a miss), hit_normal_dev float [N,R,3] (optional,
+ * NULL; world unit vector, 0 for a miss).  Fails (PRB_ERR_INVALID, with a message, before any launch) for num_rays
+ * outside 1..16384, frame outside -1..3, per_env not 0 or 1, reserved not 0, or a NULL required pointer. */
+int prb_ray_test(prb_handle* h, const prb_rays* r, const float* from_dev, const float* to_dev, int32_t* hit_collider_dev,
+                 float* hit_fraction_dev, float* hit_position_dev, float* hit_normal_dev, void* stream);
+
 /* Contact report: the contact points and forces of every env after a step, like PyBullet's getContactPoints() after
  * stepSimulation().  Off by default; prb_enable_contacts(h, 1) allocates the report (the first time) and empties it.
  * While enabled, prb_step, prb_step_host and prb_substeps (n >= 1) fill it with the contacts the LAST physics substep of

@@ -14,6 +14,7 @@
 #include <vector>
 #include "prb_reset.cuh"
 #include "prb_render.cuh"
+#include "prb_rays.cuh"
 #include "prb_contacts.cuh"
 #include "prb_dynamics.cuh"
 
@@ -620,6 +621,27 @@ int64_t prb_render_box_tests(prb_handle* h) {
   if (cudaDeviceSynchronize() != cudaSuccess) return -1;
   if (cudaMemcpy(&v, h->render_tests, sizeof(v), cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
   return (int64_t)v;
+}
+
+int prb_ray_test(prb_handle* h, const prb_rays* r, const float* from_dev, const float* to_dev, int32_t* hit_collider_dev,
+                 float* hit_fraction_dev, float* hit_position_dev, float* hit_normal_dev, void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!r) { h->err = "prb_ray_test: rays are required"; return PRB_ERR_INVALID; }
+  RayParams P;
+  const std::string why = ray_params(*r, from_dev, to_dev, hit_collider_dev, hit_fraction_dev, h->N, h->hm.n_col, &P);
+  if (!why.empty()) { h->err = "prb_ray_test: " + why; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const RayLaunch L = ray_launch(h->N, P.R);
+  if (L.small)
+    prb_ray_kernel<RAY_ENVS_SMALL><<<L.gx, L.threads, 0, s>>>(h->dm, h->state, P, from_dev, to_dev, hit_collider_dev, hit_fraction_dev,
+                                                              hit_position_dev, hit_normal_dev);
+  else
+    prb_ray_kernel<1><<<dim3(L.gx, L.gy), L.threads, 0, s>>>(h->dm, h->state, P, from_dev, to_dev, hit_collider_dev, hit_fraction_dev,
+                                                             hit_position_dev, hit_normal_dev);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  return PRB_OK;
 }
 
 int prb_enable_contacts(prb_handle* h, int32_t enable) {

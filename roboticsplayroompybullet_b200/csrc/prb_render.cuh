@@ -90,6 +90,19 @@ PRB_D float render_ndl(const RenderMem& S, const RenderParams& P, int c, float d
   return ndl;
 }
 
+// lanes of one warp: the env's state row st (read only) -> F, positions with zero velocities, then phase_fk without
+// dynamics; prb_render_kernel and prb_ray_kernel (prb_rays.cuh) place the colliders and sites from F
+PRB_D void render_load_fk(const DevModel& M, RenderFkMem& F, const float* st, int lane) {
+  if (lane < M.nd) { F.q[lane] = st[lane]; F.qd[lane] = 0.f; }
+  if (lane < M.n_free) {
+    for (int k = 0; k < 3; k++) F.fpos[lane][k] = st[5 * M.nd + 13 * lane + k];
+    for (int k = 0; k < 4; k++) F.fquat[lane][k] = st[5 * M.nd + 13 * lane + 3 + k];
+  }
+  if (lane < M.n_slide) F.sq[lane] = st[5 * M.nd + 13 * M.n_free + 2 * lane];
+  __syncwarp();
+  phase_fk(M, F, lane, false);
+}
+
 PRB_D unsigned char render_byte(float x) { return (unsigned char)floorf(255.0f * clampf(x, 0.f, 1.f) + 0.5f); }
 
 // per-collider set-up (thread c): camera -> box rotation, slab offsets of the eye, axes . light, screen rectangle
@@ -140,15 +153,7 @@ __global__ void __launch_bounds__(32 * RENDER_WARPS) prb_render_kernel(const Dev
   const size_t e = blockIdx.x;
   if (warp == 0) {
     RenderFkMem& F = S.F;
-    const float* st = state + e * M.state_stride;
-    if (lane < M.nd) { F.q[lane] = st[lane]; F.qd[lane] = 0.f; }
-    if (lane < M.n_free) {
-      for (int k = 0; k < 3; k++) F.fpos[lane][k] = st[5 * M.nd + 13 * lane + k];
-      for (int k = 0; k < 4; k++) F.fquat[lane][k] = st[5 * M.nd + 13 * lane + 3 + k];
-    }
-    if (lane < M.n_slide) F.sq[lane] = st[5 * M.nd + 13 * M.n_free + 2 * lane];
-    __syncwarp();
-    phase_fk(M, F, lane, false);
+    render_load_fk(M, F, state + e * M.state_stride, lane);
     if (lane == 0) {
       m3 Rc = ldm(P.cam);
       v3 eye = ld3(P.cam + 9);

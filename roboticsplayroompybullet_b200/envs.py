@@ -26,6 +26,9 @@ With per_env_dynamics=True every env has its own collider friction and free-body
 changeDynamics per client): change_dynamics() sets them, dynamics_device() / dynamics() return them.  With
 randomize_dynamics={field: (lo, hi)} every sampled reset first draws new values for the envs it resets (domain
 randomization).
+
+ray_test_batch_device() / ray_test_batch() cast rays against every env's collision boxes (PyBullet's rayTestBatch for all
+envs at once): the same rays in every env or rays per env, in the world or in a site of the arm.
 """
 import math
 import ctypes
@@ -119,6 +122,7 @@ class VecPlayEnv:
         self._img = None
         if self.record_images:
             self._img = torch.empty((N, self.camera.height, self.camera.width, 3), dtype=torch.uint8, device=self.device)
+        self._col_tables = None
         # contact report: allocated by the library when first enabled
         self._record_contacts = False
         self._contact_views = None
@@ -200,6 +204,17 @@ class VecPlayEnv:
         ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
         _lib.check(self.L, self._h, self.L.prb_render(self._h, ctypes.byref(cs), ctypes.c_void_p(pal.ctypes.data), ptr(rgb),
                                                      ptr(depth), ptr(seg), self._stream()))
+
+    def _body_link(self, ids):
+        """(body, link) int32 CUDA tensors of collider ids (-1 stays -1): body -1 static, 0 arm, 1.. free bodies, then
+        slide bodies; link the PyBullet link index (col_urdf_link)."""
+        t = self.torch
+        if self._col_tables is None:
+            n_col = int(self.model['n_col'])
+            self._col_tables = [t.as_tensor(np.asarray(self.model[key])[:n_col].astype(np.int32), device=self.device)
+                                for key in ('col_body', 'col_urdf_link')]
+        i = ids.clamp(min=0).long()
+        return tuple(t.where(ids >= 0, tab[i], ids) for tab in self._col_tables)
 
     def _host_copy(self):
         """Fresh arrays for the caller (the reference returns copies, environments.py:850-855): ONE copy of the pinned result
@@ -396,21 +411,45 @@ class VecPlayEnv:
                 for name, ty, k in _lib.CONTACT_FIELDS:
                     shape = (N, K) if k == 1 else (N, K, k)
                     v[name] = t.as_tensor(_DevArray(getattr(c, name), shape, self, '<' + ty), device=self.device)
-            n_col = int(self.model['n_col'])
-            tables = {key: t.as_tensor(np.asarray(self.model[key])[:n_col].astype(np.int32), device=self.device)
-                      for key in ('col_body', 'col_urdf_link')}
-            self._contact_views = (v, tables)
-        v, tables = self._contact_views
-        d = dict(v)
+            self._contact_views = v
+        d = dict(self._contact_views)
         for side in ('a', 'b'):
-            ids = v['collider_' + side]
-            for out, key in (('body_', 'col_body'), ('link_', 'col_urdf_link')):
-                d[out + side] = t.where(ids >= 0, tables[key][ids.clamp(min=0).long()], ids)
+            d['body_' + side], d['link_' + side] = self._body_link(d['collider_' + side])
         return d
 
     def contacts(self):
         """contacts_device() as numpy arrays."""
         return {k: v.cpu().numpy() for k, v in self.contacts_device().items()}
+
+    # ------------------------------------------------------------------ ray casts
+    def ray_test_batch_device(self, ray_from, ray_to, site=None, exclude_bodies=()):
+        """PyBullet's rayTestBatch(rayFromPositions, rayToPositions) in every env at once (include/prb.h, prb_ray_test): the
+        nearest collision box each segment ray_from -> ray_to hits in the current state.  ray_from, ray_to: numpy arrays or
+        CUDA tensors [R,3] (the same rays in every env) or [N,R,3] (per env), R in 1..16384, in the world (site None) or
+        in site 0..3 of the arm (0 the end effector, 1 the wrist, 2 and 3 the finger pads).  exclude_bodies: body ids
+        whose colliders cannot be hit.  Returns a dict of CUDA tensors 'collider' int32 [N,R] (-1: no hit), 'fraction'
+        float32 [N,R] (1 for no hit), 'position' and 'normal' float32 [N,R,3] (world; 0 for no hit), and 'body', 'link'
+        int32 [N,R] looked up from the collider as contacts() does.  A ray that starts inside a box hits it at fraction 0.
+        Asynchronous; ValueError for a bad shape, site or body, or a non-finite numpy input."""
+        t = self.torch
+        per_env, R, mask = check_rays(self.model, self.num_envs, ray_from, ray_to, site, exclude_bodies)
+        f, g = (t.as_tensor(x).to(self.device, t.float32).contiguous() for x in (ray_from, ray_to))
+        N = self.num_envs
+        out = {'collider': t.empty((N, R), dtype=t.int32, device=self.device),
+               'fraction': t.empty((N, R), dtype=t.float32, device=self.device),
+               'position': t.empty((N, R, 3), dtype=t.float32, device=self.device),
+               'normal': t.empty((N, R, 3), dtype=t.float32, device=self.device)}
+        r = _lib.PrbRays(R, per_env, -1 if site is None else int(site), 0, mask)
+        ptr = lambda x: ctypes.c_void_p(x.data_ptr())
+        _lib.check(self.L, self._h, self.L.prb_ray_test(self._h, ctypes.byref(r), ptr(f), ptr(g), ptr(out['collider']),
+                                                       ptr(out['fraction']), ptr(out['position']), ptr(out['normal']),
+                                                       self._stream()))
+        out['body'], out['link'] = self._body_link(out['collider'])
+        return out
+
+    def ray_test_batch(self, ray_from, ray_to, site=None, exclude_bodies=()):
+        """ray_test_batch_device() as numpy arrays."""
+        return {k: v.cpu().numpy() for k, v in self.ray_test_batch_device(ray_from, ray_to, site, exclude_bodies).items()}
 
     # ------------------------------------------------------------------ per-env dynamics
     def dynamics_device(self):
@@ -519,6 +558,35 @@ class VecPlayEnv:
         a, b, c = ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int32()
         self.L.prb_kernel_info(self._h, ctypes.byref(a), ctypes.byref(b), ctypes.byref(c))
         return {'smem_bytes_per_block': a.value, 'envs_per_block': b.value, 'regs_per_thread': c.value}
+
+
+def check_rays(model, num_envs, ray_from, ray_to, site=None, exclude_bodies=()):
+    """(per_env, R, collider_mask) of a ray_test_batch call.  ValueError unless ray_from and ray_to have one shape, [R,3]
+    or [num_envs,R,3] with R in 1..16384, site is None or 0..3, every excluded body exists, and numpy inputs are finite
+    (CUDA tensors are not read back: a ray with a non-finite endpoint is a miss)."""
+    shapes = [tuple(x.shape) for x in (ray_from, ray_to)]
+    if shapes[0] != shapes[1]:
+        raise ValueError('ray_from and ray_to must have the same shape, got %s and %s' % tuple(shapes))
+    sh = shapes[0]
+    if not ((len(sh) == 2 or (len(sh) == 3 and sh[0] == num_envs)) and sh[-1] == 3):
+        raise ValueError('rays must be [R, 3] or [num_envs=%d, R, 3], got %s' % (num_envs, sh))
+    R = sh[-2]
+    if not 1 <= R <= 16384:
+        raise ValueError('R = %d rays per env; must be in 1..16384' % R)
+    if site is not None and (isinstance(site, bool) or not isinstance(site, (int, np.integer)) or not 0 <= site <= 3):
+        raise ValueError('site must be None (world) or 0..3, got %r' % (site,))
+    for x in (ray_from, ray_to):
+        if not getattr(x, 'is_cuda', False) and not np.isfinite(np.asarray(x.cpu() if hasattr(x, 'cpu') else x, np.float64)).all():
+            raise ValueError('ray endpoints must be finite')
+    nc, nb = int(model['n_col']), int(model['n_free']) + int(model['n_slide'])
+    body = np.asarray(model['col_body'])[:nc]
+    mask = (1 << nc) - 1
+    for b in exclude_bodies:
+        if isinstance(b, bool) or not isinstance(b, (int, np.integer)) or not -1 <= b <= nb:
+            raise ValueError('exclude_bodies: %r is not a body id (-1 static, 0 arm, 1..%d)' % (b, nb))
+        for c in np.nonzero(body == b)[0]:
+            mask &= ~(1 << int(c))
+    return (1 if len(sh) == 3 else 0), R, mask
 
 
 def dynamics_ranges(spec):
