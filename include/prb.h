@@ -190,6 +190,48 @@ typedef struct prb_rays {
 int prb_ray_test(prb_handle* h, const prb_rays* r, const float* from_dev, const float* to_dev, int32_t* hit_collider_dev,
                  float* hit_fraction_dev, float* hit_position_dev, float* hit_normal_dev, void* stream);
 
+/* Closest points between collision boxes in every env, like PyBullet's getClosestPoints(bodyA, bodyB, distance[,
+ * linkIndexA, linkIndexB]) on each client.  Reads the current state (the state prb_render reads) and writes only the
+ * given arrays; asynchronous on `stream`, no host synchronisation, no allocation, exactly one kernel launch (the queries
+ * travel in its parameters).  Works with either PRB_PIPELINE.
+ *
+ * For env e and query k the candidates are every collider pair (a, b), a in mask_a, b in mask_b, a != b (two colliders of
+ * one body are a pair too).  The pair with the smallest signed distance d is reported when d <= max_distance (inclusive);
+ * ties go to the lower a, then the lower b.  Conventions of the contact report: the normal points from B towards A and
+ * position_on_a = position_on_b + distance * normal_on_b, all in the world.
+ *   * separated boxes (d > 0): d is the Euclidean distance of the two boxes, the positions a closest pair of points and
+ *     the normal (position_on_a - position_on_b) / d;
+ *   * touching or overlapping boxes (d <= 0): d = -(penetration depth), the minimum overlap over 15 separating-axis
+ *     candidates: A's 3 face axes, B's 3, the 9 edge crosses a_i x b_j (in that order; a cross with |a_i x b_j|^2 < 1e-10
+ *     is skipped).  The normal is that axis, turned towards A; on equal overlaps the lowest axis wins.  The witness is ONE
+ *     deepest point, not a manifold (prb_get_contacts gives the solver's manifolds).  Its candidates, in this order: for
+ *     an edge cross the point of A's supporting edge nearest B's supporting edge as position_on_a; A's deepest vertex
+ *     (its support along -normal) as position_on_a; B's deepest vertex (its support along the normal) as position_on_b;
+ *     two points found by projecting alternately onto A's and B's supporting features (vertex, edge or face; a box axis
+ *     with |normal . axis| < 1e-4 spans the feature), from B's or from A's feature centre.  The other point always
+ *     follows from position_on_a = position_on_b + distance * normal, and the first candidate whose two points lie
+ *     nearest their boxes and supporting planes (L1) wins; supports take sign(0) = +.
+ * Recalled from PyBullet, not verified against a PyBullet run: `distance` is an inclusive bound, the sign and direction
+ * conventions above.  PyBullet returns one point per pair of shapes within reach; this call returns only the nearest
+ * pair of each query. */
+typedef struct prb_closest_query {
+  uint64_t mask_a, mask_b;   /* colliders of side A and side B (bit c: collider c; bits >= n_col ignored) */
+} prb_closest_query;
+typedef struct prb_closest {
+  int32_t num_queries;       /* Q, 1..64 */
+  int32_t reserved;          /* must be 0 */
+  float max_distance;        /* PyBullet's `distance`: finite, >= 0 (m) */
+  int32_t reserved2;         /* must be 0 */
+} prb_closest;
+/* queries_host: Q host structs.  Outputs (device, indexed in 64 bits): collider_a_dev, collider_b_dev int32 [N,Q] and
+ * distance_dev float [N,Q] (required), position_on_a_dev, position_on_b_dev, normal_on_b_dev float [N,Q,3] (optional,
+ * NULL).  No pair within reach: colliders -1, distance +inf, positions and normal 0.  Fails (PRB_ERR_INVALID, with a
+ * message, before any launch) for num_queries outside 1..64, a reserved field not 0, a non-finite or negative
+ * max_distance, or a NULL required pointer. */
+int prb_closest_points(prb_handle* h, const prb_closest* q, const prb_closest_query* queries_host, int32_t* collider_a_dev,
+                       int32_t* collider_b_dev, float* distance_dev, float* position_on_a_dev, float* position_on_b_dev,
+                       float* normal_on_b_dev, void* stream);
+
 /* Contact report: the contact points and forces of every env after a step, like PyBullet's getContactPoints() after
  * stepSimulation().  Off by default; prb_enable_contacts(h, 1) allocates the report (the first time) and empties it.
  * While enabled, prb_step, prb_step_host and prb_substeps (n >= 1) fill it with the contacts the LAST physics substep of

@@ -15,6 +15,7 @@
 #include "prb_reset.cuh"
 #include "prb_render.cuh"
 #include "prb_rays.cuh"
+#include "prb_closest.cuh"
 #include "prb_contacts.cuh"
 #include "prb_dynamics.cuh"
 
@@ -639,6 +640,22 @@ int prb_ray_test(prb_handle* h, const prb_rays* r, const float* from_dev, const 
   else
     prb_ray_kernel<1><<<dim3(L.gx, L.gy), L.threads, 0, s>>>(h->dm, h->state, P, from_dev, to_dev, hit_collider_dev, hit_fraction_dev,
                                                              hit_position_dev, hit_normal_dev);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  return PRB_OK;
+}
+
+int prb_closest_points(prb_handle* h, const prb_closest* q, const prb_closest_query* queries_host, int32_t* collider_a_dev,
+                       int32_t* collider_b_dev, float* distance_dev, float* position_on_a_dev, float* position_on_b_dev,
+                       float* normal_on_b_dev, void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!q) { h->err = "prb_closest_points: the call struct is required"; return PRB_ERR_INVALID; }
+  ClosestParams P;
+  const std::string why = closest_params(*q, queries_host, collider_a_dev, collider_b_dev, distance_dev, h->N, h->hm.n_col, &P);
+  if (!why.empty()) { h->err = "prb_closest_points: " + why; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  prb_closest_kernel<true><<<closest_blocks(h->N), 32 * CLOSEST_ENVS, 0, (cudaStream_t)stream>>>(
+      h->dm, h->state, P, collider_a_dev, collider_b_dev, distance_dev, position_on_a_dev, position_on_b_dev, normal_on_b_dev);
   h->launches++;
   CK(h, cudaGetLastError());
   return PRB_OK;

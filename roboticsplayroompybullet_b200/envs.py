@@ -29,6 +29,9 @@ randomization).
 
 ray_test_batch_device() / ray_test_batch() cast rays against every env's collision boxes (PyBullet's rayTestBatch for all
 envs at once): the same rays in every env or rays per env, in the world or in a site of the arm.
+
+closest_points_device() / closest_points() give the nearest pair of collision boxes between two bodies or links in every
+env (PyBullet's getClosestPoints for all envs at once): signed distance, witness points and normal.
 """
 import math
 import ctypes
@@ -451,6 +454,37 @@ class VecPlayEnv:
         """ray_test_batch_device() as numpy arrays."""
         return {k: v.cpu().numpy() for k, v in self.ray_test_batch_device(ray_from, ray_to, site, exclude_bodies).items()}
 
+    # ------------------------------------------------------------------ closest points
+    def closest_points_device(self, queries, max_distance):
+        """PyBullet's getClosestPoints(bodyA, bodyB, distance[, linkIndexA, linkIndexB]) in every env at once (include/prb.h,
+        prb_closest_points).  queries: a list of Q in 1..64 pairs (side_a, side_b); a side is a body id (all its colliders)
+        or a (body, link) tuple, the ids of contacts(): body -1 static scene, 0 arm, 1.. free bodies, then slide bodies;
+        link the PyBullet link index.  For each query the nearest collider pair (a, b), a != b, with signed distance
+        <= max_distance (m, inclusive).  Returns a dict of CUDA tensors 'collider_a', 'collider_b', 'body_a', 'body_b',
+        'link_a', 'link_b' int32 [N,Q] (-1: no pair within reach), 'distance' float32 [N,Q] (< 0: penetration; inf: no
+        pair), 'position_on_a', 'position_on_b', 'normal_on_b' float32 [N,Q,3] (world; the normal points from B to A;
+        0 for no pair).  Asynchronous; ValueError for an unknown body or link, no or more than 64 queries, or a
+        non-finite or negative max_distance."""
+        t = self.torch
+        qs, md = check_closest(self.model, queries, max_distance)
+        N, Q = self.num_envs, len(qs)
+        out = {k: t.empty((N, Q), dtype=t.int32, device=self.device) for k in ('collider_a', 'collider_b')}
+        out['distance'] = t.empty((N, Q), dtype=t.float32, device=self.device)
+        for k in ('position_on_a', 'position_on_b', 'normal_on_b'):
+            out[k] = t.empty((N, Q, 3), dtype=t.float32, device=self.device)
+        arr = (_lib.PrbClosestQuery * Q)(*[_lib.PrbClosestQuery(a, b) for a, b in qs])
+        c = _lib.PrbClosest(Q, 0, md, 0)
+        ptr = lambda x: ctypes.c_void_p(x.data_ptr())
+        _lib.check(self.L, self._h, self.L.prb_closest_points(self._h, ctypes.byref(c), arr, *[ptr(out[k]) for k in (
+            'collider_a', 'collider_b', 'distance', 'position_on_a', 'position_on_b', 'normal_on_b')], self._stream()))
+        for side in ('a', 'b'):
+            out['body_' + side], out['link_' + side] = self._body_link(out['collider_' + side])
+        return out
+
+    def closest_points(self, queries, max_distance):
+        """closest_points_device() as numpy arrays."""
+        return {k: v.cpu().numpy() for k, v in self.closest_points_device(queries, max_distance).items()}
+
     # ------------------------------------------------------------------ per-env dynamics
     def dynamics_device(self):
         """The per-env dynamics table (include/prb.h, prb_dynamics) as zero-copy CUDA tensors: 'lateral_friction',
@@ -587,6 +621,38 @@ def check_rays(model, num_envs, ray_from, ray_to, site=None, exclude_bodies=()):
         for c in np.nonzero(body == b)[0]:
             mask &= ~(1 << int(c))
     return (1 if len(sh) == 3 else 0), R, mask
+
+
+def check_closest(model, queries, max_distance):
+    """([(mask_a, mask_b)] collider masks, max_distance) of a closest_points call.  ValueError unless there are 1..64
+    queries, each a pair of sides, a side a body id or a (body, link) tuple with at least one collider, and max_distance
+    is finite and >= 0."""
+    queries = list(queries)
+    if not 1 <= len(queries) <= 64:
+        raise ValueError('closest_points needs 1..64 queries, got %d' % len(queries))
+    nc = int(model['n_col'])
+    body = np.asarray(model['col_body'])[:nc]
+
+    def side_mask(side):
+        if isinstance(side, tuple) and len(side) == 2:
+            cols = dynamics_target(model, *side)[0]
+        elif isinstance(side, (int, np.integer)) and not isinstance(side, bool):
+            cols = np.nonzero(body == int(side))[0]
+            if len(cols) == 0:
+                raise ValueError('no collider has body %r' % (side,))
+        else:
+            raise ValueError('a query side is a body id or a (body, link) tuple, got %r' % (side,))
+        return sum(1 << int(c) for c in cols)
+
+    qs = []
+    for q in queries:
+        if not (isinstance(q, (tuple, list)) and len(q) == 2):
+            raise ValueError('a query is a pair (side_a, side_b), got %r' % (q,))
+        qs.append((side_mask(q[0]), side_mask(q[1])))
+    md = float(max_distance)
+    if not (math.isfinite(md) and md >= 0.0):
+        raise ValueError('max_distance must be finite and >= 0, got %r' % (max_distance,))
+    return qs, md
 
 
 def dynamics_ranges(spec):
