@@ -232,6 +232,50 @@ int prb_closest_points(prb_handle* h, const prb_closest* q, const prb_closest_qu
                        int32_t* collider_b_dev, float* distance_dev, float* position_on_a_dev, float* position_on_b_dev,
                        float* normal_on_b_dev, void* stream);
 
+/* The arm's Jacobians, joint-space mass matrix and inverse dynamics in every env, like PyBullet's calculateJacobian,
+ * calculateMassMatrix and calculateInverseDynamics on each client.  Reads the current state and the caller's arrays and
+ * writes only the given outputs; asynchronous on `stream`, no host synchronisation, no allocation, exactly one kernel
+ * launch (the points travel in its parameters).  Works with either PRB_PIPELINE.
+ *
+ * The arm (body 0) only: its nd DoF (12 UR5, 9 Panda) in the compiled model's link order, with the model's fixed base.
+ * Free and slide bodies are not covered.  Each env is evaluated at q and qd from q_dev / qd_dev (float [N,nd], device)
+ * when given, each from the env's state row when NULL; qdd from qdd_dev when given, 0 when NULL.  The state is never
+ * written.
+ *
+ * Points (num_points P in 0..16): site = -1: local_position in the frame of model arm link `link` (0..nd-1), the link
+ * (joint) frame after the joint's motion; site = 0..3: local_position in site s's frame (as prb_ray_test's frames: 0 the
+ * end effector, 1 the wrist, 2 and 3 the finger pads), and link must be -1.
+ * Outputs (device, float, indexed in 64 bits; each optional, at least one given):
+ *   * jacobian_dev [N,P,6,nd]: rows 0-2 linear, 3-5 angular, world frame.  Column j for a point x on link l is 0 unless
+ *     j is an ancestor-or-self of l; revolute j: (a_j x (x - p_j), a_j); prismatic j: (a_j, 0), with a_j the joint's
+ *     world axis and p_j its link frame origin;
+ *   * point_position_dev [N,P,3]: the world position of each point;
+ *   * point_velocity_dev [N,P,6]: J qd (linear, angular), the point's world velocity;
+ *   * mass_matrix_dev [N,nd,nd]: M(q), symmetric bit for bit; the step's own arithmetic (composite rigid bodies);
+ *   * tau_dev [N,nd]: tau = M(q) qdd + h(q, qd), h the Coriolis, centrifugal and gravity term (the step's recursive
+ *     Newton-Euler bias, before joint damping).  Joint damping, motors, limits, gears, contacts and link damping are
+ *     not included.  qdd = 0 gives the bias h; qd = qdd = 0 the gravity-holding torques.  Without qdd_dev tau is h.
+ * Fails (PRB_ERR_INVALID, with a message, before any launch) for num_points outside 0..16, points without a point
+ * output or a point output without points, a NULL points_host with points, a link outside 0..nd-1 for site -1, a site
+ * outside -1..3 or a site with link != -1, a reserved field not 0, or no output at all.
+ * Recalled from PyBullet, not verified against a PyBullet run: PyBullet's localPosition is relative to the link's centre
+ * of mass (its inertial frame), here to the link frame or a site frame; PyBullet's inverse dynamics is believed to
+ * leave out joint damping, as here.  The columns here are in the model's link order; the Python layer
+ * (arm_dof_joints) maps them to PyBullet joint indices. */
+typedef struct prb_arm_point {
+  int32_t link;              /* model arm link 0..nd-1 (site -1), or -1 (a site point) */
+  int32_t site;              /* -1: the link frame; 0..3: a site frame */
+  float local_position[3];   /* m, in that frame */
+  int32_t reserved;          /* must be 0 */
+} prb_arm_point;
+typedef struct prb_arm_query {
+  int32_t num_points;        /* P, 0..16 */
+  int32_t reserved;          /* must be 0 */
+} prb_arm_query;
+int prb_arm_dynamics(prb_handle* h, const prb_arm_query* q, const prb_arm_point* points_host, const float* q_dev,
+                     const float* qd_dev, const float* qdd_dev, float* jacobian_dev, float* point_position_dev,
+                     float* point_velocity_dev, float* mass_matrix_dev, float* tau_dev, void* stream);
+
 /* Contact report: the contact points and forces of every env after a step, like PyBullet's getContactPoints() after
  * stepSimulation().  Off by default; prb_enable_contacts(h, 1) allocates the report (the first time) and empties it.
  * While enabled, prb_step, prb_step_host and prb_substeps (n >= 1) fill it with the contacts the LAST physics substep of

@@ -16,6 +16,7 @@
 #include "prb_render.cuh"
 #include "prb_rays.cuh"
 #include "prb_closest.cuh"
+#include "prb_arm.cuh"
 #include "prb_contacts.cuh"
 #include "prb_dynamics.cuh"
 
@@ -656,6 +657,23 @@ int prb_closest_points(prb_handle* h, const prb_closest* q, const prb_closest_qu
   DevGuard guard(h->device);
   prb_closest_kernel<true><<<closest_blocks(h->N), 32 * CLOSEST_ENVS, 0, (cudaStream_t)stream>>>(
       h->dm, h->state, P, collider_a_dev, collider_b_dev, distance_dev, position_on_a_dev, position_on_b_dev, normal_on_b_dev);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  return PRB_OK;
+}
+
+int prb_arm_dynamics(prb_handle* h, const prb_arm_query* q, const prb_arm_point* points_host, const float* q_dev,
+                     const float* qd_dev, const float* qdd_dev, float* jacobian_dev, float* point_position_dev,
+                     float* point_velocity_dev, float* mass_matrix_dev, float* tau_dev, void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!q) { h->err = "prb_arm_dynamics: the call struct is required"; return PRB_ERR_INVALID; }
+  ArmParams P;
+  const std::string why = arm_params(*q, points_host, jacobian_dev, point_position_dev, point_velocity_dev, mass_matrix_dev,
+                                     tau_dev, h->N, h->hm.nd, h->hm.site_link, &P);
+  if (!why.empty()) { h->err = "prb_arm_dynamics: " + why; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  prb_arm_kernel<<<arm_blocks(h->N), 32 * ARM_ENVS, 0, (cudaStream_t)stream>>>(
+      h->dm, h->state, P, q_dev, qd_dev, qdd_dev, jacobian_dev, point_position_dev, point_velocity_dev, mass_matrix_dev, tau_dev);
   h->launches++;
   CK(h, cudaGetLastError());
   return PRB_OK;

@@ -462,43 +462,48 @@ PRB_D void phase_fk(const DevModel& M, WM& W, int lane, bool dynamics, const flo
   __syncwarp();
 }
 
-// bias forces tau_j and mass-matrix row j (lane = joint j), by direct sums over subtree(j)
+// Joint j's bias torque tau_j (the velocity-product and gravity term h_j of tau = M qdd + h) and mass-matrix row j
+// (W.Mm[j][k] and W.Mm[k][j], k <= j), by direct sums over subtree(j).  put(tau_j) runs where the step stores its
+// generalized force, so that phase_crba and prb_arm_kernel share this arithmetic and its order.
+template <class WM, class PUT>
+PRB_D void crba_joint(const DevModel& M, WM& W, int j, PUT put) {
+  const int nd = M.nd;
+  const bool rev = M.jtype[j] == 0;
+  const v3 aj = ld3(W.la[j]), pj = ld3(W.lp[j]);
+  float tau = 0;
+  v3 P = V3(0, 0, 0), L = V3(0, 0, 0);
+  unsigned mask = M.sub_mask[j];
+#pragma unroll 1
+  for (int i = j; i < nd; i++) {
+    if (!((mask >> i) & 1u)) continue;
+    v3 ci = ld3(W.lc[i]), fi = ld3(W.lf[i]), ni = ld3(W.ln[i]);
+    v3 rc = ci - pj;
+    tau += rev ? dot(aj, ni + cross(rc, fi)) : dot(aj, fi);
+    float mi = M.mass[i];
+    v3 ui = rev ? cross(aj, rc) : aj;
+    v3 pm = ui * mi;
+    P = P + pm;
+    L = L + cross(rc, pm);
+    if (rev) L = L + symmul(W.lIw[i], aj);
+  }
+  put(tau);
+  unsigned anc = M.anc_mask[j];
+#pragma unroll 1
+  for (int k = 0; k <= j; k++) {
+    float val = 0.f;
+    if ((anc >> k) & 1u) {
+      v3 ak = ld3(W.la[k]);
+      val = M.jtype[k] == 0 ? dot(ak, L + cross(pj - ld3(W.lp[k]), P)) : dot(ak, P);
+    }
+    W.Mm[j][k] = val;
+    W.Mm[k][j] = val;
+  }
+}
+
+// generalized bias forces W.Q = -tau - jdamp qd and the mass matrix W.Mm (lane = joint j)
 template <class WM>
 PRB_D void phase_crba(const DevModel& M, WM& W, int lane) {
-  const int nd = M.nd;
-  if (lane < nd) {
-    const int j = lane;
-    const bool rev = M.jtype[j] == 0;
-    const v3 aj = ld3(W.la[j]), pj = ld3(W.lp[j]);
-    float tau = 0;
-    v3 P = V3(0, 0, 0), L = V3(0, 0, 0);
-    unsigned mask = M.sub_mask[j];
-#pragma unroll 1
-    for (int i = j; i < nd; i++) {
-      if (!((mask >> i) & 1u)) continue;
-      v3 ci = ld3(W.lc[i]), fi = ld3(W.lf[i]), ni = ld3(W.ln[i]);
-      v3 rc = ci - pj;
-      tau += rev ? dot(aj, ni + cross(rc, fi)) : dot(aj, fi);
-      float mi = M.mass[i];
-      v3 ui = rev ? cross(aj, rc) : aj;
-      v3 pm = ui * mi;
-      P = P + pm;
-      L = L + cross(rc, pm);
-      if (rev) L = L + symmul(W.lIw[i], aj);
-    }
-    W.Q[j] = -tau - M.jdamp[j] * W.qd[j];
-    unsigned anc = M.anc_mask[j];
-#pragma unroll 1
-    for (int k = 0; k <= j; k++) {
-      float val = 0.f;
-      if ((anc >> k) & 1u) {
-        v3 ak = ld3(W.la[k]);
-        val = M.jtype[k] == 0 ? dot(ak, L + cross(pj - ld3(W.lp[k]), P)) : dot(ak, P);
-      }
-      W.Mm[j][k] = val;
-      W.Mm[k][j] = val;
-    }
-  }
+  if (lane < M.nd) crba_joint(M, W, lane, [&](float tau) { W.Q[lane] = -tau - M.jdamp[lane] * W.qd[lane]; });
   __syncwarp();
 }
 

@@ -32,6 +32,11 @@ envs at once): the same rays in every env or rays per env, in the world or in a 
 
 closest_points_device() / closest_points() give the nearest pair of collision boxes between two bodies or links in every
 env (PyBullet's getClosestPoints for all envs at once): signed distance, witness points and normal.
+
+calculate_jacobian_device(), calculate_mass_matrix_device() and calculate_inverse_dynamics_device() (and their numpy
+twins) give the arm's point Jacobians, joint-space mass matrix and inverse dynamics in every env (PyBullet's
+calculateJacobian, calculateMassMatrix and calculateInverseDynamics for all envs at once); arm_dof_joints maps their
+columns to PyBullet joint indices.
 """
 import math
 import ctypes
@@ -485,6 +490,72 @@ class VecPlayEnv:
         """closest_points_device() as numpy arrays."""
         return {k: v.cpu().numpy() for k, v in self.closest_points_device(queries, max_distance).items()}
 
+    # ------------------------------------------------------------------ arm dynamics
+    @property
+    def arm_dof_joints(self):
+        """PyBullet joint index of each arm DoF, i.e. of each column of the Jacobians, the mass matrix and tau (the model's
+        link order; the link ids contacts() reports for body 0)."""
+        return np.asarray(self.model['arm_urdf_index'])[:int(self.model['nd'])].copy()
+
+    def _arm_dynamics(self, points, q, qd, qdd, want):
+        """One prb_arm_dynamics call that asks for the outputs in `want` only: dict of CUDA tensors."""
+        t = self.torch
+        N, nd, P = self.num_envs, int(self.model['nd']), len(points)
+        shapes = {'jacobian': (N, P, 6, nd), 'position': (N, P, 3), 'velocity': (N, P, 6), 'mass_matrix': (N, nd, nd),
+                  'tau': (N, nd)}
+        out = {k: t.empty(shapes[k], dtype=t.float32, device=self.device) for k in want}
+        ins = [None if x is None else t.as_tensor(x).to(self.device, t.float32).contiguous() for x in (q, qd, qdd)]
+        pts = (_lib.PrbArmPoint * max(P, 1))(*[_lib.PrbArmPoint(l, s, (ctypes.c_float * 3)(*o), 0) for l, s, o in points])
+        ptr = lambda x: None if x is None else ctypes.c_void_p(x.data_ptr())
+        _lib.check(self.L, self._h, self.L.prb_arm_dynamics(
+            self._h, ctypes.byref(_lib.PrbArmQuery(P, 0)), pts, *[ptr(x) for x in ins],
+            *[ptr(out.get(k)) for k in ('jacobian', 'position', 'velocity', 'mass_matrix', 'tau')], self._stream()))
+        return out
+
+    def calculate_jacobian_device(self, local_positions=((0.0, 0.0, 0.0),), link=None, site=0, q=None, qd=None):
+        """PyBullet's calculateJacobian(arm, linkIndex, localPosition, q, qd, qdd) in every env at once, for P in 1..16
+        points (include/prb.h, prb_arm_dynamics).  The points are local_positions [P,3] (m) in the frame of arm link
+        `link` (a PyBullet link index of arm_dof_joints; pass site=None) or of site `site` (0 the end effector, 1 the
+        wrist, 2 and 3 the finger pads).  q, qd: numpy arrays or CUDA tensors [N, nd]; each defaults to the env's state.
+        Returns a dict of CUDA tensors 'linear' and 'angular' float32 [N,P,3,nd] (world frame; columns in arm_dof_joints
+        order), 'position' [N,P,3] (world) and 'velocity' [N,P,6] (J qd: linear, angular).  Asynchronous; ValueError for
+        a bad shape, an unknown link or site, both or neither of link and site, or a non-finite numpy input."""
+        points = check_arm_points(self.model, local_positions, link, site)
+        check_arm_inputs(self.num_envs, int(self.model['nd']), q=q, qd=qd)
+        out = self._arm_dynamics(points, q, qd, None, ('jacobian', 'position', 'velocity'))
+        J = out.pop('jacobian')
+        out['linear'], out['angular'] = J[:, :, :3], J[:, :, 3:]
+        return out
+
+    def calculate_jacobian(self, local_positions=((0.0, 0.0, 0.0),), link=None, site=0, q=None, qd=None):
+        """calculate_jacobian_device() as numpy arrays."""
+        return {k: v.cpu().numpy() for k, v in self.calculate_jacobian_device(local_positions, link, site, q, qd).items()}
+
+    def calculate_mass_matrix_device(self, q=None):
+        """PyBullet's calculateMassMatrix(arm, q) in every env at once: the joint-space inertia M(q) of the arm, a CUDA
+        tensor float32 [N, nd, nd] (symmetric; rows and columns in arm_dof_joints order), the matrix the step uses.
+        q: numpy array or CUDA tensor [N, nd], default the env's state.  Asynchronous; ValueError for a bad shape or a
+        non-finite numpy input."""
+        check_arm_inputs(self.num_envs, int(self.model['nd']), q=q)
+        return self._arm_dynamics([], q, None, None, ('mass_matrix',))['mass_matrix']
+
+    def calculate_mass_matrix(self, q=None):
+        """calculate_mass_matrix_device() as a numpy array."""
+        return self.calculate_mass_matrix_device(q).cpu().numpy()
+
+    def calculate_inverse_dynamics_device(self, qdd=None, q=None, qd=None):
+        """PyBullet's calculateInverseDynamics(arm, q, qd, qdd) in every env at once: tau = M(q) qdd + h(q, qd), h the
+        Coriolis, centrifugal and gravity term, without joint damping, motors, limits, gears or contacts; a CUDA tensor
+        float32 [N, nd] (arm_dof_joints order; N m for revolute, N for prismatic DoF).  qdd default 0 (the bias h);
+        q, qd default the env's state; each a numpy array or CUDA tensor [N, nd].  Asynchronous; ValueError for a bad
+        shape or a non-finite numpy input."""
+        check_arm_inputs(self.num_envs, int(self.model['nd']), q=q, qd=qd, qdd=qdd)
+        return self._arm_dynamics([], q, qd, qdd, ('tau',))['tau']
+
+    def calculate_inverse_dynamics(self, qdd=None, q=None, qd=None):
+        """calculate_inverse_dynamics_device() as a numpy array."""
+        return self.calculate_inverse_dynamics_device(qdd, q, qd).cpu().numpy()
+
     # ------------------------------------------------------------------ per-env dynamics
     def dynamics_device(self):
         """The per-env dynamics table (include/prb.h, prb_dynamics) as zero-copy CUDA tensors: 'lateral_friction',
@@ -653,6 +724,40 @@ def check_closest(model, queries, max_distance):
     if not (math.isfinite(md) and md >= 0.0):
         raise ValueError('max_distance must be finite and >= 0, got %r' % (max_distance,))
     return qs, md
+
+
+def check_arm_points(model, local_positions, link=None, site=0):
+    """[(model link, site, (x, y, z))] prb_arm_point fields of a calculate_jacobian call.  ValueError unless exactly one of
+    link (a PyBullet link index of the arm, arm_urdf_index) and site (0..3) is given and local_positions is a finite
+    [P,3] with P in 1..16."""
+    if (link is None) == (site is None):
+        raise ValueError('give exactly one of link and site, got link=%r, site=%r' % (link, site))
+    x = np.asarray(local_positions.cpu() if hasattr(local_positions, 'cpu') else local_positions, np.float64)
+    if x.ndim != 2 or x.shape[1] != 3 or not 1 <= x.shape[0] <= 16:
+        raise ValueError('local_positions must be [P, 3] with P in 1..16, got shape %s' % (x.shape,))
+    if not np.isfinite(x).all():
+        raise ValueError('local_positions must be finite')
+    if site is not None:
+        if isinstance(site, bool) or not isinstance(site, (int, np.integer)) or not 0 <= site <= 3:
+            raise ValueError('site must be 0..3, got %r' % (site,))
+        return [(-1, int(site), tuple(r)) for r in x]
+    urdf = list(np.asarray(model['arm_urdf_index'])[:int(model['nd'])])
+    if isinstance(link, bool) or not isinstance(link, (int, np.integer)) or int(link) not in urdf:
+        raise ValueError('link must be a PyBullet link index of the arm %s, got %r' % ([int(u) for u in urdf], link))
+    return [(urdf.index(int(link)), -1, tuple(r)) for r in x]
+
+
+def check_arm_inputs(num_envs, nd, **arrays):
+    """ValueError unless every given array (numpy or CUDA tensor; None: not given) is [num_envs, nd] and, for numpy,
+    finite (CUDA tensors are not read back)."""
+    for name, x in arrays.items():
+        if x is None:
+            continue
+        shape = tuple(x.shape) if hasattr(x, 'shape') else np.shape(x)
+        if shape != (num_envs, nd):
+            raise ValueError('%s must be [num_envs=%d, nd=%d], got %s' % (name, num_envs, nd, shape))
+        if not getattr(x, 'is_cuda', False) and not np.isfinite(np.asarray(x.cpu() if hasattr(x, 'cpu') else x, np.float64)).all():
+            raise ValueError('%s must be finite' % name)
 
 
 def dynamics_ranges(spec):
