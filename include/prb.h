@@ -276,10 +276,86 @@ int prb_arm_dynamics(prb_handle* h, const prb_arm_query* q, const prb_arm_point*
                      const float* qd_dev, const float* qdd_dev, float* jacobian_dev, float* point_position_dev,
                      float* point_velocity_dev, float* mass_matrix_dev, float* tau_dev, void* stream);
 
+/* Link and joint states of every env, like PyBullet's getLinkStates(computeLinkVelocity=1, computeForwardKinematics=1),
+ * getBasePositionAndOrientation, getBaseVelocity and getJointStates on each client.  Reads the current state only and
+ * writes only the given outputs; asynchronous on `stream`, no host synchronisation, no allocation, exactly one kernel
+ * launch.  Works with either PRB_PIPELINE.
+ *
+ * body_dev float [N,K,13], K = nd + n_free + n_slide: one row per body frame, pos[3] | quat[4] (x, y, z, w) | linear
+ * velocity[3] | angular velocity[3], all in the world frame (the layout of a free body in the state row).  Rows, in order:
+ *   * the arm's nd links in the compiled model's link order (the columns of prb_arm_dynamics);
+ *   * the n_free free bodies (block, drawer): their 13 state floats, bit for bit, in either frame;
+ *   * the n_slide slide bodies (door, button, dial): the body frame after its joint's motion; the linear velocity of a
+ *     prismatic body, or the angular velocity of a revolute one, is sqd times its world joint axis, the other part 0.
+ *     The compiled model keeps no centre-of-mass offset for them, so both frames are the same.
+ * q->frame 0 reports each arm link's link (joint) frame, PyBullet's worldLinkFramePosition / Orientation; 1 its inertial
+ * frame, PyBullet's linkWorldPosition / Orientation: the link frame moved to the link's centre of mass (the compiled
+ * model keeps the inertia in the link frame, so the orientation is the link frame's).  Velocities are those of the
+ * chosen frame's origin: the COM frame's linear velocity is v + w x (c - p).  Orientations come from the link's
+ * rotation matrix (Shepperd's method, mat_to_quat), so their sign is not tied to any earlier reading.
+ * joint_q_dev, joint_qd_dev float [N, nd + n_slide]: the arm's DoF (model link order), then the slide joints (door,
+ * button, dial), straight from the state row.  Each output is optional (NULL); at least one is required.
+ * Fails (PRB_ERR_INVALID, with a message, before any launch) for frame not 0 or 1, reserved not 0, or no output.
+ * Recalled from PyBullet, not verified against a PyBullet run: which of PyBullet's two frames carries the "link frame"
+ * name, and that computeLinkVelocity reports the COM frame's velocity.  Applied joint torques and reaction forces are
+ * not reported. */
+typedef struct prb_body_query {
+  int32_t frame;             /* 0: link (joint) frames; 1: centre-of-mass (inertial) frames */
+  int32_t reserved;          /* must be 0 */
+} prb_body_query;
+int prb_body_states(prb_handle* h, const prb_body_query* q, float* body_dev, float* joint_q_dev, float* joint_qd_dev,
+                    void* stream);
+
+/* Masked writes of joint positions and velocities and free-body poses and velocities, like PyBullet's resetJointState,
+ * resetBasePositionAndOrientation and resetBaseVelocity on each client.  Asynchronous on `stream`, no host
+ * synchronisation, no allocation.
+ *
+ * Selection: bit j of joint_positions / joint_velocities is column j of [0, nd + n_slide) (the columns of
+ * prb_body_states' joint arrays: arm DoF, then slide joints); bit b of free_poses / free_velocities is free body b of
+ * [0, n_free).  Inputs use the read layouts: joint_q_dev, joint_qd_dev float [N, nd + n_slide], body_dev float [N,K,13]
+ * of which only the selected words of the free-body rows (pos | quat, or linear | angular velocity) are read, so a
+ * prb_body_states read, an edit and this call round-trip.  Only envs with mask_dev[e] != 0 (uint8 [N]; NULL: all) are
+ * written.
+ *
+ * Positions and velocities are written exactly; a written quaternion is divided by its norm in fp32 (unfused, correctly
+ * rounded: n = sqrt(((x x + y y) + z z) + w w), q / n).  Motor targets, gains and impulse limits, the goal, the reset
+ * counter and the per-env dynamics table are left alone, as PyBullet's resetJointState leaves motors alone.  A masked env
+ * whose selected inputs hold a non-finite value, or a quaternion of norm < 1e-6 (or beyond fp32), is left completely
+ * unchanged.  status_dev (uint8 [N], optional) gets 0 for an env not masked, 1 written, 2 rejected.
+ *
+ * In the same call, for the written envs only: the contact report (when enabled) is emptied, and the output buffers are
+ * refreshed as prb_observe does (the masked setup launch), so that for them the call gives the same bits as editing
+ * the rows, prb_set_state, then prb_observe.  Other envs keep their state and outputs bit for bit.  Launches: the write
+ * kernel, the report clear when the report is enabled, one setup launch.
+ *
+ * No constraint is enforced at the write: a write that breaks one (the UR5 gripper's gear and mimic rows, joint limits,
+ * the drawer's rail) is allowed, and the next physics substep's joint rows pull it back, as in PyBullet.
+ * Fails (PRB_ERR_INVALID, with a message, before any launch) for bits at or beyond nd + n_slide or n_free, no bit set,
+ * a selected input that is NULL, or reserved not 0. */
+typedef struct prb_state_write {
+  uint32_t joint_positions;   /* bit j: write q of column j */
+  uint32_t joint_velocities;  /* bit j: write qd of column j */
+  uint32_t free_poses;        /* bit b: write position and orientation of free body b */
+  uint32_t free_velocities;   /* bit b: write linear and angular velocity of free body b */
+  int32_t reserved;           /* must be 0 */
+} prb_state_write;
+int prb_write_state(prb_handle* h, const prb_state_write* w, const float* joint_q_dev, const float* joint_qd_dev,
+                    const float* body_dev, const uint8_t* mask_dev, uint8_t* status_dev, void* stream);
+
+/* Device-side snapshots, like PyBullet's saveState / restoreState for every env.  prb_save_state copies the state
+ * [N, state_stride] (prb_buffers.state_stride) into dst_dev with one cudaMemcpyAsync.  prb_restore_state copies the
+ * rows of the envs of mask_dev (uint8 [N]; NULL: all) back from src_dev (one launch), empties their contact report when
+ * it is enabled and refreshes their output buffers as prb_observe does.  Restored rows equal the saved rows bit for bit;
+ * the other rows are not touched.  The per-env dynamics table is not part of a snapshot (as with prb_set_state).
+ * Asynchronous on `stream`.  Fails (PRB_ERR_INVALID) for a NULL dst_dev / src_dev. */
+int prb_save_state(prb_handle* h, float* dst_dev, void* stream);
+int prb_restore_state(prb_handle* h, const float* src_dev, const uint8_t* mask_dev, void* stream);
+
 /* Contact report: the contact points and forces of every env after a step, like PyBullet's getContactPoints() after
  * stepSimulation().  Off by default; prb_enable_contacts(h, 1) allocates the report (the first time) and empties it.
  * While enabled, prb_step, prb_step_host and prb_substeps (n >= 1) fill it with the contacts the LAST physics substep of
- * the call solved; prb_reset, prb_reset_to and prb_set_state empty it (count 0) for every env whose state they change;
+ * the call solved; prb_reset, prb_reset_to, prb_set_state, prb_write_state and prb_restore_state empty it (count 0)
+ * for every env whose state they change;
  * prb_observe, prb_set_goal and prb_render leave it unchanged.  With PRB_PIPELINE=fused enabling fails (PRB_ERR_INVALID).
  *
  * Env e has count[e] (0..max_contacts = 64) contacts: those after manifold reduction (<= 4 per pair of collision

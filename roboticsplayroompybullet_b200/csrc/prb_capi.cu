@@ -17,6 +17,7 @@
 #include "prb_rays.cuh"
 #include "prb_closest.cuh"
 #include "prb_arm.cuh"
+#include "prb_state.cuh"
 #include "prb_contacts.cuh"
 #include "prb_dynamics.cuh"
 
@@ -67,6 +68,7 @@ struct prb_handle {
   int contacts = 0;                // 1: prb_step / prb_substeps refresh the contact report
   float* dyn = nullptr;            // per-env dynamics table (prb_stream.cuh layout; allocated when first enabled)
   int dynamics = 0;                // 1: every setup launch reads the table instead of the model
+  unsigned char* written = nullptr;   // [N] envs the last prb_write_state wrote (its clear and observe mask)
   std::string err;
 };
 
@@ -318,6 +320,8 @@ int prb_create(const prb_model* model, const prb_config* cfg, prb_handle** out) 
   CK(h, cudaMemset(h->O.ovf_env, 0, N));
   CK(h, cudaMalloc(&h->pending, N));
   CK(h, cudaMemset(h->pending, 0, N));
+  CK(h, cudaMalloc(&h->written, N));
+  CK(h, cudaMemset(h->written, 0, N));
   CK(h, cudaMalloc(&h->reset_ctl, sizeof(int) * 2 * N));
   CK(h, cudaMemset(h->reset_ctl, 0, sizeof(int) * 2 * N));
   CK(h, cudaMalloc(&h->n_pending, sizeof(int)));
@@ -367,7 +371,7 @@ int prb_destroy(prb_handle* h) {
   DevGuard guard(h->device);
   cudaDeviceSynchronize();
   cudaFree(h->dm); cudaFree(h->state); cudaFree(h->out); cudaFree(h->action_stage); cudaFree(h->O.overflow); cudaFree(h->O.dbg); cudaFree(h->sbuf);
-  cudaFree(h->O.ovf_env); cudaFree(h->pending); cudaFree(h->reset_ctl); cudaFree(h->n_pending); cudaFree(h->elist[0]); cudaFree(h->elist[1]);
+  cudaFree(h->O.ovf_env); cudaFree(h->pending); cudaFree(h->written); cudaFree(h->reset_ctl); cudaFree(h->n_pending); cudaFree(h->elist[0]); cudaFree(h->elist[1]);
   if (h->n_pending_host) cudaFreeHost(h->n_pending_host);
   if (h->out_stage) { cudaFreeHost(h->out_stage); for (int c = 0; c < prb_handle::OUT_CHUNKS; c++) cudaEventDestroy(h->ev_chunk[c]); }
   for (int k = 0; k < ARM_NCLASS; k++) {
@@ -677,6 +681,61 @@ int prb_arm_dynamics(prb_handle* h, const prb_arm_query* q, const prb_arm_point*
   h->launches++;
   CK(h, cudaGetLastError());
   return PRB_OK;
+}
+
+int prb_body_states(prb_handle* h, const prb_body_query* q, float* body_dev, float* joint_q_dev, float* joint_qd_dev,
+                    void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!q) { h->err = "prb_body_states: the call struct is required"; return PRB_ERR_INVALID; }
+  const std::string why = body_query_check(*q, body_dev, joint_q_dev, joint_qd_dev);
+  if (!why.empty()) { h->err = "prb_body_states: " + why; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  prb_body_state_kernel<<<state_blocks(h->N), 32 * STATE_ENVS, 0, (cudaStream_t)stream>>>(h->dm, h->state, h->N, q->frame, body_dev,
+                                                                                        joint_q_dev, joint_qd_dev);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  return PRB_OK;
+}
+
+int prb_write_state(prb_handle* h, const prb_state_write* w, const float* joint_q_dev, const float* joint_qd_dev,
+                    const float* body_dev, const uint8_t* mask_dev, uint8_t* status_dev, void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!w) { h->err = "prb_write_state: the call struct is required"; return PRB_ERR_INVALID; }
+  StateWrite P;
+  const std::string why = state_write_params(*w, joint_q_dev, joint_qd_dev, body_dev, h->hm.nd, h->hm.n_free, h->hm.n_slide, &P);
+  if (!why.empty()) { h->err = "prb_write_state: " + why; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  prb_write_state_kernel<<<state_blocks(h->N), 32 * STATE_ENVS, 0, s>>>(h->dm, h->state, h->N, P, joint_q_dev, joint_qd_dev, body_dev,
+                                                                       mask_dev, status_dev, h->written);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  const int rc = clear_contacts(h, h->written, s);
+  if (rc != PRB_OK) return rc;
+  return run_step(h, 0, 1, s, h->written);
+}
+
+int prb_save_state(prb_handle* h, float* dst_dev, void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!dst_dev) { h->err = "prb_save_state: dst_dev is required"; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  CK(h, cudaMemcpyAsync(dst_dev, h->state, sizeof(float) * (size_t)h->N * h->hm.state_stride, cudaMemcpyDeviceToDevice,
+                        (cudaStream_t)stream));
+  return PRB_OK;
+}
+
+int prb_restore_state(prb_handle* h, const float* src_dev, const uint8_t* mask_dev, void* stream) {
+  if (!h) return PRB_ERR_INVALID;
+  if (!src_dev) { h->err = "prb_restore_state: src_dev is required"; return PRB_ERR_INVALID; }
+  DevGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t words = (int64_t)h->N * h->hm.state_stride;
+  prb_restore_state_kernel<<<(unsigned)((words + 255) / 256), 256, 0, s>>>(h->state, src_dev, mask_dev, words, h->hm.state_stride);
+  h->launches++;
+  CK(h, cudaGetLastError());
+  const int rc = clear_contacts(h, mask_dev, s);
+  if (rc != PRB_OK) return rc;
+  return run_step(h, 0, 1, s, mask_dev);
 }
 
 int prb_enable_contacts(prb_handle* h, int32_t enable) {

@@ -37,6 +37,12 @@ calculate_jacobian_device(), calculate_mass_matrix_device() and calculate_invers
 twins) give the arm's point Jacobians, joint-space mass matrix and inverse dynamics in every env (PyBullet's
 calculateJacobian, calculateMassMatrix and calculateInverseDynamics for all envs at once); arm_dof_joints maps their
 columns to PyBullet joint indices.
+
+body_states_device() / joint_states_device() read every link, free body and slide body frame and every joint of every
+env (PyBullet's getLinkStates, getBasePositionAndOrientation, getBaseVelocity, getJointStates);
+reset_joint_states_device() / reset_base_states_device() write them for masked envs (resetJointState,
+resetBasePositionAndOrientation, resetBaseVelocity); save_state_device() / restore_state_device() keep and restore
+device-side snapshots (saveState / restoreState).  Each has a numpy twin.
 """
 import math
 import ctypes
@@ -556,6 +562,167 @@ class VecPlayEnv:
         """calculate_inverse_dynamics_device() as a numpy array."""
         return self.calculate_inverse_dynamics_device(qdd, q, qd).cpu().numpy()
 
+    # ------------------------------------------------------------------ link and joint states
+    @property
+    def body_state_ids(self):
+        """(body, link) of each row of body_states_device(), an int32 array [K, 2]: the arm's links (body 0, PyBullet link
+        index, arm_dof_joints order), the free bodies (1.., link -1), then the slide bodies (door, button, dial; link -1),
+        the ids of contacts() and change_dynamics()."""
+        return state_ids(self.model)[0]
+
+    @property
+    def joint_state_ids(self):
+        """(body, joint) of each column of joint_states_device(), an int32 array [nd + n_slide, 2]: the arm's DoF (body 0,
+        PyBullet joint index, arm_dof_joints), then each slide body's one joint (joint 0 of that body)."""
+        return state_ids(self.model)[1]
+
+    def _body_states(self, frame):
+        t = self.torch
+        fr = check_frame(frame)
+        body = t.empty((self.num_envs, len(self.body_state_ids), 13), dtype=t.float32, device=self.device)
+        _lib.check(self.L, self._h, self.L.prb_body_states(self._h, ctypes.byref(_lib.PrbBodyQuery(fr, 0)),
+                                                          ctypes.c_void_p(body.data_ptr()), None, None, self._stream()))
+        return body
+
+    def body_states_device(self, frame='link'):
+        """PyBullet's getLinkStates(computeLinkVelocity=1), getBasePositionAndOrientation and getBaseVelocity for every body
+        frame of every env at once (include/prb.h, prb_body_states): a dict of views of one float32 CUDA tensor [N,K,13],
+        'position' [N,K,3], 'orientation' [N,K,4] (x, y, z, w), 'linear_velocity' and 'angular_velocity' [N,K,3], all in
+        the world frame; row k is body_state_ids[k].  frame 'link': each arm link's link (joint) frame, 'com': its
+        centre-of-mass frame (velocities are those of the frame's origin); free and slide bodies are the same in both.
+        Asynchronous; ValueError for an unknown frame."""
+        body = self._body_states(frame)
+        return {'position': body[..., 0:3], 'orientation': body[..., 3:7], 'linear_velocity': body[..., 7:10],
+                'angular_velocity': body[..., 10:13]}
+
+    def body_states(self, frame='link'):
+        """body_states_device() as numpy arrays."""
+        return {k: v.cpu().numpy() for k, v in self.body_states_device(frame).items()}
+
+    def joint_states_device(self):
+        """PyBullet's getJointStates (positions and velocities) for every env at once: 'position' and 'velocity', float32
+        CUDA tensors [N, nd + n_slide]; column j is joint_state_ids[j].  Asynchronous."""
+        t = self.torch
+        q, qd = (t.empty((self.num_envs, len(self.joint_state_ids)), dtype=t.float32, device=self.device) for _ in range(2))
+        _lib.check(self.L, self._h, self.L.prb_body_states(self._h, ctypes.byref(_lib.PrbBodyQuery(0, 0)), None,
+                                                          ctypes.c_void_p(q.data_ptr()), ctypes.c_void_p(qd.data_ptr()),
+                                                          self._stream()))
+        return {'position': q, 'velocity': qd}
+
+    def joint_states(self):
+        """joint_states_device() as numpy arrays."""
+        return {k: v.cpu().numpy() for k, v in self.joint_states_device().items()}
+
+    def _mask_dev(self, mask):
+        if mask is None:
+            return None
+        t = self.torch
+        m = mask if isinstance(mask, t.Tensor) else t.as_tensor(np.asarray(mask))
+        if tuple(m.shape) != (self.num_envs,):
+            raise ValueError('mask must be [num_envs=%d], got %s' % (self.num_envs, tuple(m.shape)))
+        return m.to(self.device, t.uint8).contiguous()
+
+    def _write_state(self, w, jq, jqd, body, mask):
+        """One prb_write_state call; returns the status tensor (uint8 [N]: 0 not masked, 1 written, 2 rejected)."""
+        t = self.torch
+        status = t.empty(self.num_envs, dtype=t.uint8, device=self.device)
+        self._w_keep = (jq, jqd, body, mask)        # the call is asynchronous: inputs live until the next write
+        ptr = lambda x: None if x is None else ctypes.c_void_p(x.data_ptr())
+        _lib.check(self.L, self._h, self.L.prb_write_state(self._h, ctypes.byref(w), ptr(jq), ptr(jqd), ptr(body), ptr(mask),
+                                                          ptr(status), self._stream()))
+        return status
+
+    def reset_joint_states_device(self, position, velocity=None, joints=None, mask=None):
+        """PyBullet's resetJointState(body, joint, targetValue, targetVelocity) for every env of `mask` (uint8 / bool [N];
+        None: all) at once.  joints: a list of (body, joint) ids of joint_state_ids (None: every column); position and
+        velocity: numpy arrays or CUDA tensors [N, len(joints)] or [len(joints)] (the same in every env); a missing
+        velocity is 0.  Motors, goals and dynamics are left alone; the written envs' contact report is emptied and their
+        observation refreshed.  Returns the status, a uint8 CUDA tensor [N] (0 not masked, 1 written, 2 rejected: a
+        non-finite CUDA input leaves its env unchanged).  Asynchronous; ValueError for an unknown or repeated joint, a bad
+        shape or a non-finite numpy input."""
+        t = self.torch
+        cols = check_joints(self.model, joints)
+        N, nj = self.num_envs, len(self.joint_state_ids)
+        vals = [check_state_value(name, x, N, len(cols)) for name, x in (('position', position), ('velocity', velocity))]
+        jq, jqd = (t.zeros((N, nj), dtype=t.float32, device=self.device) for _ in range(2))
+        ci = t.as_tensor(cols, dtype=t.long, device=self.device)
+        for dst, v in zip((jq, jqd), vals):
+            if v is not None:
+                dst[:, ci] = t.as_tensor(v).to(self.device, t.float32).expand(N, len(cols))
+        bits = sum(1 << c for c in cols)
+        return self._write_state(_lib.PrbStateWrite(bits, bits, 0, 0, 0), jq, jqd, None, self._mask_dev(mask))
+
+    def reset_joint_states(self, position, velocity=None, joints=None, mask=None):
+        """reset_joint_states_device(); returns the status as a numpy array."""
+        return self.reset_joint_states_device(position, velocity, joints, mask).cpu().numpy()
+
+    def reset_base_states_device(self, body, position=None, orientation=None, linear_velocity=None, angular_velocity=None,
+                                 mask=None):
+        """PyBullet's resetBasePositionAndOrientation and resetBaseVelocity of free body `body` (1..n_free, the ids of
+        contacts()) for every env of `mask` (None: all) at once.  Each part is a numpy array or CUDA tensor [N, k] or [k]
+        (position 3, orientation 4 as x, y, z, w, normalised in fp32 by the library; velocities 3, world frame); a part
+        left out keeps its current value (read with one body_states call).  The written envs' contact report is emptied
+        and their observation refreshed.  Returns the status, a uint8 CUDA tensor [N] (0 not masked, 1 written, 2
+        rejected: a non-finite value or a quaternion of norm < 1e-6 in a CUDA input).  Asynchronous; ValueError for a
+        body that is not a free body, no part given, a bad shape, or a non-finite numpy input or zero numpy quaternion."""
+        nf, nd = int(self.model['n_free']), int(self.model['nd'])
+        if isinstance(body, bool) or not isinstance(body, (int, np.integer)) or not 1 <= body <= nf:
+            raise ValueError('body must be a free body id 1..%d, got %r' % (nf, body))
+        parts = {'position': (position, 0, 3), 'orientation': (orientation, 3, 7), 'linear_velocity': (linear_velocity, 7, 10),
+                 'angular_velocity': (angular_velocity, 10, 13)}
+        N = self.num_envs
+        vals = {k: (check_state_value(k, x, N, b - a), a, b) for k, (x, a, b) in parts.items() if x is not None}
+        if not vals:
+            raise ValueError('give at least one of position, orientation, linear_velocity, angular_velocity')
+        t = self.torch
+        cur = self._body_states('link')
+        row = nd + int(body) - 1
+        for v, a, b in vals.values():
+            cur[:, row, a:b] = t.as_tensor(v).to(self.device, t.float32).expand(N, b - a)
+        bit = 1 << (int(body) - 1)
+        pose = bit if ('position' in vals or 'orientation' in vals) else 0
+        vel = bit if ('linear_velocity' in vals or 'angular_velocity' in vals) else 0
+        return self._write_state(_lib.PrbStateWrite(0, 0, pose, vel, 0), None, None, cur, self._mask_dev(mask))
+
+    def reset_base_states(self, body, position=None, orientation=None, linear_velocity=None, angular_velocity=None,
+                          mask=None):
+        """reset_base_states_device(); returns the status as a numpy array."""
+        return self.reset_base_states_device(body, position, orientation, linear_velocity, angular_velocity, mask).cpu().numpy()
+
+    def save_state_device(self):
+        """PyBullet's saveState for every env at once: a float32 CUDA tensor [N, state_stride], a copy of the state
+        (without the per-env dynamics table).  Asynchronous."""
+        t = self.torch
+        snap = t.empty((self.num_envs, self.buffers.state_stride), dtype=t.float32, device=self.device)
+        _lib.check(self.L, self._h, self.L.prb_save_state(self._h, ctypes.c_void_p(snap.data_ptr()), self._stream()))
+        return snap
+
+    def save_state(self):
+        """save_state_device() as a numpy array."""
+        return self.save_state_device().cpu().numpy()
+
+    def restore_state_device(self, saved, mask=None):
+        """PyBullet's restoreState for every env of `mask` (uint8 / bool [N]; None: all) at once, from a save_state_device()
+        snapshot (a CUDA tensor or numpy array [N, state_stride]): the rows come back bit for bit, the contact report of
+        the restored envs is emptied and their observation refreshed.  Asynchronous; ValueError for a bad shape or a
+        non-finite numpy snapshot."""
+        t = self.torch
+        shape = (self.num_envs, self.buffers.state_stride)
+        if tuple(saved.shape) != shape:
+            raise ValueError('saved must be [num_envs, state_stride] = %s, got %s' % (shape, tuple(saved.shape)))
+        if not isinstance(saved, t.Tensor) and not np.isfinite(np.asarray(saved, np.float32)[:, :self.buffers.state_dim]).all():
+            raise ValueError('saved must be finite')
+        src = t.as_tensor(saved).to(self.device, t.float32).contiguous()
+        m = self._mask_dev(mask)
+        self._w_keep = (src, m)
+        _lib.check(self.L, self._h, self.L.prb_restore_state(self._h, ctypes.c_void_p(src.data_ptr()),
+                                                            None if m is None else ctypes.c_void_p(m.data_ptr()), self._stream()))
+
+    def restore_state(self, saved, mask=None):
+        """restore_state_device() from a numpy snapshot; synchronises the stream."""
+        self.restore_state_device(saved, mask)
+        self.torch.cuda.current_stream(self.device).synchronize()
+
     # ------------------------------------------------------------------ per-env dynamics
     def dynamics_device(self):
         """The per-env dynamics table (include/prb.h, prb_dynamics) as zero-copy CUDA tensors: 'lateral_friction',
@@ -758,6 +925,61 @@ def check_arm_inputs(num_envs, nd, **arrays):
             raise ValueError('%s must be [num_envs=%d, nd=%d], got %s' % (name, num_envs, nd, shape))
         if not getattr(x, 'is_cuda', False) and not np.isfinite(np.asarray(x.cpu() if hasattr(x, 'cpu') else x, np.float64)).all():
             raise ValueError('%s must be finite' % name)
+
+
+def state_ids(model):
+    """(body_state_ids [K, 2], joint_state_ids [nd + n_slide, 2]) of a compiled model, int32: rows of prb_body_states are
+    the arm's links (0, PyBullet link index), the free bodies (1.., -1) and the slide bodies (1 + n_free.., -1); columns of
+    its joint arrays the arm's DoF (0, PyBullet joint index) and each slide body's one joint (body, 0)."""
+    nd, nf, ns = int(model['nd']), int(model['n_free']), int(model['n_slide'])
+    urdf = [int(u) for u in np.asarray(model['arm_urdf_index'])[:nd]]
+    bodies = [(0, u) for u in urdf] + [(1 + b, -1) for b in range(nf)] + [(1 + nf + s, -1) for s in range(ns)]
+    joints = [(0, u) for u in urdf] + [(1 + nf + s, 0) for s in range(ns)]
+    return np.array(bodies, np.int32).reshape(-1, 2), np.array(joints, np.int32).reshape(-1, 2)
+
+
+def check_frame(frame):
+    """prb_body_query.frame of 'link' (0) or 'com' (1); ValueError otherwise."""
+    if frame not in ('link', 'com'):
+        raise ValueError("frame must be 'link' or 'com', got %r" % (frame,))
+    return 0 if frame == 'link' else 1
+
+
+def check_joints(model, joints):
+    """Column indices of a list of (body, joint) ids of joint_state_ids (None: every column).  ValueError for an unknown
+    or repeated id, or an empty list."""
+    ids = [tuple(int(v) for v in r) for r in state_ids(model)[1]]
+    if joints is None:
+        return list(range(len(ids)))
+    cols = []
+    for j in joints:
+        if not (isinstance(j, (tuple, list)) and len(j) == 2 and all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in j)):
+            raise ValueError('a joint is a (body, joint) id, got %r' % (j,))
+        if tuple(int(v) for v in j) not in ids:
+            raise ValueError('unknown joint %r (joint_state_ids: %s)' % (tuple(j), ids))
+        cols.append(ids.index(tuple(int(v) for v in j)))
+    if not cols or len(set(cols)) != len(cols):
+        raise ValueError('joints must be a non-empty list without repeats, got %r' % (list(joints),))
+    return cols
+
+
+def check_state_value(name, x, N, k):
+    """A state write input (numpy array or CUDA tensor; None: not given) of shape [N, k] or [k].  ValueError for another
+    shape and, for numpy, a non-finite value or an orientation of norm < 1e-6 (CUDA tensors are not read back: the
+    library rejects such an env)."""
+    if x is None:
+        return None
+    shape = tuple(x.shape) if hasattr(x, 'shape') else np.shape(x)
+    if shape not in ((N, k), (k,)):
+        raise ValueError('%s must be [num_envs=%d, %d] or [%d], got %s' % (name, N, k, k, shape))
+    if getattr(x, 'is_cuda', False):
+        return x
+    a = np.asarray(x.cpu() if hasattr(x, 'cpu') else x, np.float64)
+    if not np.isfinite(a).all():
+        raise ValueError('%s must be finite' % name)
+    if name == 'orientation' and (np.linalg.norm(a.reshape(-1, 4), axis=1) < 1e-6).any():
+        raise ValueError('orientation quaternions must have a norm >= 1e-6')
+    return np.ascontiguousarray(a, np.float32)
 
 
 def dynamics_ranges(spec):

@@ -57,6 +57,15 @@ class PrbArmQuery(ctypes.Structure):
     _fields_ = [('num_points', ctypes.c_int32), ('reserved', ctypes.c_int32)]
 
 
+class PrbBodyQuery(ctypes.Structure):
+    _fields_ = [('frame', ctypes.c_int32), ('reserved', ctypes.c_int32)]
+
+
+class PrbStateWrite(ctypes.Structure):
+    _fields_ = [('joint_positions', ctypes.c_uint32), ('joint_velocities', ctypes.c_uint32), ('free_poses', ctypes.c_uint32),
+                ('free_velocities', ctypes.c_uint32), ('reserved', ctypes.c_int32)]
+
+
 # prb_contacts: the contact report's device arrays; (name, element type, per-contact components) in struct order
 CONTACT_FIELDS = [('collider_a', 'i4', 1), ('collider_b', 'i4', 1), ('position_on_a', 'f4', 3), ('position_on_b', 'f4', 3),
                   ('normal_on_b', 'f4', 3), ('distance', 'f4', 1), ('normal_force', 'f4', 1), ('lateral_friction_1', 'f4', 1),
@@ -88,6 +97,7 @@ SYMBOLS = ['prb_create', 'prb_destroy', 'prb_reset', 'prb_reset_rounds', 'prb_re
            'prb_get_buffers', 'prb_compute_reward', 'prb_get_state', 'prb_set_state', 'prb_step_host',
            'prb_enable_kernel_timing', 'prb_last_kernel_ms', 'prb_last_tier_ms', 'prb_launch_count', 'prb_overflow_count', 'prb_debug_usage', 'prb_kernel_info', 'prb_render', 'prb_render_box_tests',
            'prb_ray_test', 'prb_closest_points', 'prb_arm_dynamics',
+           'prb_body_states', 'prb_write_state', 'prb_save_state', 'prb_restore_state',
            'prb_enable_contacts', 'prb_get_contacts', 'prb_enable_dynamics', 'prb_get_dynamics', 'prb_randomize_dynamics',
            'prb_last_error',
            'prb_version']
@@ -135,6 +145,10 @@ def load():
     L.prb_ray_test.argtypes = [vp, ctypes.POINTER(PrbRays), vp, vp, vp, vp, vp, vp, vp]
     L.prb_closest_points.argtypes = [vp, ctypes.POINTER(PrbClosest), ctypes.POINTER(PrbClosestQuery), vp, vp, vp, vp, vp, vp, vp]
     L.prb_arm_dynamics.argtypes = [vp, ctypes.POINTER(PrbArmQuery), ctypes.POINTER(PrbArmPoint), vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.prb_body_states.argtypes = [vp, ctypes.POINTER(PrbBodyQuery), vp, vp, vp, vp]
+    L.prb_write_state.argtypes = [vp, ctypes.POINTER(PrbStateWrite), vp, vp, vp, vp, vp, vp]
+    L.prb_save_state.argtypes = [vp, vp, vp]
+    L.prb_restore_state.argtypes = [vp, vp, vp, vp]
     L.prb_enable_contacts.argtypes = [vp, i32]
     L.prb_get_contacts.argtypes = [vp, ctypes.POINTER(PrbContacts)]
     L.prb_enable_dynamics.argtypes = [vp, i32]
