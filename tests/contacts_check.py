@@ -109,9 +109,9 @@ def compare(model, Oracle, rep, states, geom_tol, rng=None, n_pert=8, f32_probe=
     moves by a comparable amount (1 / COND_K of it) when its input state is perturbed by one fp32 ulp.  With f32_probe,
     also when the oracle's fp32 restatement (Oracle(f32=True)) deviates from the fp64 oracle by 1 / COND_K of it: over
     the 12 substeps of a full step the rounding of the whole computation, not only of the input, sets the spread.  Returns
-    {n, cond (envs accepted by these rules), bad (list of (env, reason)), worst_geom, worst_force}."""
+    {n, cond (envs accepted by these rules), cond_envs (which), bad (list of (env, reason)), worst_geom, worst_force}."""
     rng = rng if rng is not None else np.random.default_rng(0)
-    res = {'n': len(states), 'cond': 0, 'bad': [], 'worst_geom': 0.0, 'worst_force': 0.0}
+    res = {'n': len(states), 'cond': 0, 'cond_envs': [], 'bad': [], 'worst_geom': 0.0, 'worst_force': 0.0}
     for j, (i, row, adv) in enumerate(states):
         o = Oracle(model)
         o.state[:] = np.asarray(row, np.float64)
@@ -164,6 +164,7 @@ def compare(model, Oracle, rep, states, geom_tol, rng=None, n_pert=8, f32_probe=
             ok = set_changes or diff <= COND_K * spread_force
         if ok:
             res['cond'] += 1
+            res['cond_envs'].append(i)
         else:
             res['bad'].append((i, reason))
     return res

@@ -26,6 +26,9 @@ ANG_TOL = 1e-3        # rad (Euler entries of 'observation')
 VEL_ABS, VEL_REL = 3e-2, 1e-2   # the pose tolerance seen as a speed: 1e-4 m per 1/300 s substep = 3e-2 m/s (rad/s)
 COND_K = 8.0          # |cuda - oracle| <= COND_K x (spread of the oracle under 1-ulp input perturbations)
 DIAL_PERIOD = 2.0 / 2.2   # scenes.py:342-343: (q mod 2) / 2.2 wraps at q = 0 -> compare modulo the period
+# compile-time defines of the small-stage build (csrc/prb_stream.cuh): arm-island classes of 104-120 q and a free-body stage
+# of 16 q, so that most arm records are read from the class buffer in place; emulated and nvcc builds use the same list
+SMALL_STAGE = ['ARM_CAPQ0=104', 'ARM_CAPQ1=108', 'ARM_CAPQ2=112', 'ARM_CAPQ3=116', 'ARM_CAPQ4=120', 'PGS_STAGE_F=16']
 
 
 def random_actions(rng, n, env_id):

@@ -9,13 +9,12 @@ import pytest
 import contacts_check as cc
 from emu_contacts import ContactSim
 from emu_lib import EmuSim
-from helpers import random_actions
+from helpers import SMALL_STAGE as SMALL, random_actions
 from oracle.oracle import Oracle
 from roboticsplayroompybullet_b200.model import load_model
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 PLAY = 'UR5PlayAbsRPY1Obj-v0'
-SMALL = ['ARM_CAPQ0=104', 'ARM_CAPQ1=108', 'ARM_CAPQ2=112', 'ARM_CAPQ3=116', 'ARM_CAPQ4=120', 'PGS_STAGE_F=16']
 
 
 def _rollout_states(env_id, n=3, steps=3, seed=5):

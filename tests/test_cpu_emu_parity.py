@@ -161,7 +161,8 @@ def test_emu_records_read_in_place_when_stage_is_small():
     stage of 16 q) every grasp lands in the last class and most of its records are read from the class buffer in
     place; the grasp sequence must give the SAME states as the normal build, bit for bit."""
     from emu_lib import lib_variant
-    small = lib_variant('smallstage', ['ARM_CAPQ0=104', 'ARM_CAPQ1=108', 'ARM_CAPQ2=112', 'ARM_CAPQ3=116', 'ARM_CAPQ4=120', 'PGS_STAGE_F=16'])
+    from helpers import SMALL_STAGE
+    small = lib_variant('smallstage', SMALL_STAGE)
     m = load_model('UR5PlayAbsRPY1Obj-v0')
     a_sim, b_sim, o = EmuSim(m, 1, seed=3), EmuSim(m, 1, seed=3, library=small), Oracle(m, seed=3)
     o.reset()
@@ -322,3 +323,27 @@ def test_emu_more_than_32_contacts():
     res = compare_step(m, {k: de[k] for k in OBS_KEYS}, de['reward'][:, 0], {'is_success': de['is_success'][:, 0]}, outs,
                        g['state'], g['action'], Oracle)
     assert res['bad_pose'] == 0 and res['bad_vel'] == 0 and res['bad_reward'] == 0 and res['stiff'] <= 2, res
+
+
+def test_emu_fused_pipeline_counts_each_overflowing_env_once():
+    """The fused A/B kernel holds 32 overlapping pairs and 32 contacts per env (prb_kernels.cuh, CfgL): every one of the 17
+    many-contact states exceeds that in some substep of its step, and the capacity counter goes up by exactly one per env
+    step, however many substeps dropped something.  The split pipeline drops nothing on the same states."""
+    import os
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'many_contacts.npz'))
+    m = load_model('UR5PlayAbsRPY1Obj-v0')
+    n = len(g['state'])
+    sd = Oracle(m).state_dim
+    deltas = {}
+    for fused in (1, 0):
+        sim = EmuSim(m, n, seed=1)
+        sim.state[:, :sd] = g['state']
+        ov0 = sim.L.emu_overflow()
+        sim.L.emu_set_fused(fused)
+        try:
+            de = sim.step(g['action'])
+        finally:
+            sim.L.emu_set_fused(0)
+        deltas[fused] = sim.L.emu_overflow() - ov0
+        assert all(np.isfinite(v).all() for v in de.values()) and np.isfinite(sim.state).all()
+    assert deltas == {1: n, 0: 0}, deltas
