@@ -30,6 +30,8 @@
 #define __noinline__
 #define __restrict__
 #define __launch_bounds__(...)
+#define __maxnreg__(n)
+#define __grid_constant__
 #define __shared__ static
 #define __constant__ static
 
@@ -185,13 +187,19 @@ static inline unsigned __ballot_sync(unsigned, int pred) {
 static inline int __any_sync(unsigned m, int p) { return __ballot_sync(m, p) != 0; }
 static inline int __all_sync(unsigned m, int p) { return __ballot_sync(m, !p) == 0; }
 static inline int __popc(unsigned x) { return __builtin_popcount(x); }
+static inline int __popcll(unsigned long long x) { return __builtin_popcountll(x); }
 static inline int __ffs(int x) { return __builtin_ffs(x); }
+static inline int __ffsll(long long x) { return __builtin_ffsll(x); }
 static inline int __clz(int x) { return x == 0 ? 32 : __builtin_clz((unsigned)x); }
 template <class T> static inline T atomicAdd(T* p, T v) { T o = *p; *p = o + v; return o; }
 template <class T> static inline T __ldg(const T* p) { return *p; }
 static inline float rsqrtf(float x) { return 1.0f / sqrtf(x); }
 static inline float __frcp_rn(float x) { return 1.0f / x; }
 static inline float __fdividef(float a, float b) { return a / b; }
+static inline float __fmul_rn(float a, float b) { return a * b; }
+static inline float __fadd_rn(float a, float b) { return a + b; }
+static inline float __fsqrt_rn(float a) { return sqrtf(a); }
+static inline float __fdiv_rn(float a, float b) { return a / b; }
 static inline void sincosf_emu(float x, float* s, float* c) { *s = sinf(x); *c = cosf(x); }
 #ifndef sincosf
 #define sincosf(x, s, c) sincosf_emu(x, s, c)

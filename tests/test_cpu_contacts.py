@@ -1,13 +1,12 @@
 """The contact report (include/prb.h prb_contacts) on the CPU SIMT emulator: the step pipeline in report mode
-(tests/emu/contacts_emu.cpp) against the fp64 oracle's contacts and impulses, the read-in-place solver path, and the
-physics a report must satisfy without an oracle."""
+(EmuSim(report=True), tests/emu/prb_emu.cpp) against the fp64 oracle's contacts and impulses, the read-in-place solver
+path, and the physics a report must satisfy without an oracle."""
 import os
 
 import numpy as np
 import pytest
 
 import contacts_check as cc
-from emu_contacts import ContactSim
 from emu_lib import EmuSim
 from helpers import SMALL_STAGE as SMALL, random_actions
 from oracle.oracle import Oracle
@@ -46,7 +45,7 @@ def _inputs():
 
 
 def _run(m, states, actions, full_step):
-    sim = ContactSim(m, len(states))
+    sim = EmuSim(m, len(states), report=True)
     sim.set_state(states)
     if full_step:
         sim.step(actions)
@@ -104,7 +103,7 @@ def test_report_read_in_place_bit_identical():
     blk = o.state[60:63].copy()
     act = lambda z, g: np.array([[blk[0], blk[1], z, 0, 0, 0, g]], np.float32)
     seq = [act(-0.01, -1)] * 14 + [act(-0.01, 1)] * 8 + [act(0.15, 1)] * 4
-    sims = [ContactSim(m, 1), ContactSim(m, 1, tag='smallstage', defines=SMALL), ContactSim(m, 1, report=False)]
+    sims = [EmuSim(m, 1, report=True), EmuSim(m, 1, report=True, tag='smallstage', defines=SMALL), EmuSim(m, 1)]
     ref = EmuSim(m, 1, seed=3)
     for s in sims + [ref]:
         s.state[0, :o.state_dim] = o.state.astype(np.float32)
@@ -133,7 +132,7 @@ def test_resting_block_carries_its_weight(env_id):
     n = 4
     sim = EmuSim(m, n, seed=13)
     sim.reset()
-    cs = ContactSim(m, n)
+    cs = EmuSim(m, n, report=True)
     cs.set_state(sim.state)
     cs.substeps(1)
     rep = cs.contacts()
@@ -157,7 +156,7 @@ def test_clear_mask_empties_only_the_masked_envs():
     """prb_reset / prb_reset_to / prb_set_state's emptying of the report: the masked envs get count 0 and padding, the
     others keep their report bit for bit."""
     m, states, actions = _rollout_states(PLAY, n=2, steps=2)
-    cs = ContactSim(m, len(states))
+    cs = EmuSim(m, len(states), report=True)
     cs.set_state(states)
     cs.substeps(1)
     before = cs.contacts()

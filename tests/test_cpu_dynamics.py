@@ -1,6 +1,6 @@
 """Per-env dynamics (include/prb.h prb_dynamics) on the CPU SIMT emulator: the setup kernel with the table
-(tests/emu/dynamics_emu.cpp) against itself without it, against emulator runs and oracle runs of models patched to each
-env's values, against physics that shares no code with the kernels, and the randomization kernel."""
+(EmuSim(table=...), tests/emu/prb_emu.cpp) against itself without it, against emulator runs and oracle runs of models
+patched to each env's values, against physics that shares no code with the kernels, and the randomization kernel."""
 import ctypes
 import os
 import subprocess
@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 import contacts_check as cc
-from emu_dynamics import FIELDS, MODEL_FIELD, DynSim, model_table
+from emu_dynamics import FIELDS, MODEL_FIELD, model_table
 from emu_lib import EmuSim
 from helpers import OBS_KEYS, compare_step, oracle_step_from, random_actions
 from oracle.oracle import Oracle
@@ -81,7 +81,7 @@ def test_table_with_model_values_is_bit_identical():
     no table, over full steps of every input set."""
     for m, states, actions in _inputs():
         N = len(states)
-        off, on = DynSim(m, N), DynSim(m, N, table=model_table(m, N))
+        off, on = EmuSim(m, N), EmuSim(m, N, table=model_table(m, N))
         for s in (off, on):
             s.set_state(states)
         for _ in range(2):
@@ -96,14 +96,14 @@ def test_per_env_equals_per_model():
     for m, states, actions in _inputs():
         sets = _param_sets(m)
         K, N = len(sets), len(states)
-        sim = DynSim(m, N, table=_table(sets, N))
+        sim = EmuSim(m, N, table=_table(sets, N))
         sim.set_state(states)
         out = sim.step(actions)
         for k in range(K):
             idx = np.arange(k, N, K)
             if len(idx) == 0:
                 continue
-            ref = DynSim(_patched(m, sets[k]), len(idx))
+            ref = EmuSim(_patched(m, sets[k]), len(idx))
             ref.set_state(states[idx])
             ro = ref.step(actions[idx])
             assert np.array_equal(sim.state[idx], ref.state), k
@@ -132,7 +132,7 @@ def test_oracle_parity_one_step():
     for m, states, actions in _inputs():
         sets = _param_sets(m)
         N = len(states)
-        sim = DynSim(m, N, table=_table(sets, N))
+        sim = EmuSim(m, N, table=_table(sets, N))
         sim.set_state(states)
         out = sim.step(actions)
         res = _oracle_check(m, sets, states, actions, out, rng)
@@ -148,7 +148,7 @@ def test_oracle_parity_rollout():
     base = EmuSim(m, N, seed=21)
     base.reset()
     sd = base.state_dim
-    sim = DynSim(m, N, table=_table(sets, N))
+    sim = EmuSim(m, N, table=_table(sets, N))
     sim.set_state(base.state[:, :sd])
     rng, crng = np.random.default_rng(4), np.random.default_rng(1)
     stiff = 0
@@ -171,7 +171,7 @@ def _block_on_table(m, N, table, report=False):
     st[:, f0:f0 + 3] = [0.0, 0.18, st[0, f0 + 2]]
     st[:, f0 + 3:f0 + 7] = [0, 0, 0, 1]
     st[:, f0 + 7:f0 + 13] = 0
-    sim = DynSim(m, N, table=table, report=report)
+    sim = EmuSim(m, N, report=report, table=table)
     sim.set_state(st)
     sim.substeps(60)
     return sim, f0
@@ -239,7 +239,7 @@ def test_free_flight_with_per_env_damping():
     t = model_table(m, N)
     t['linear_damping'][:, 0] = damp[:, 0]
     t['angular_damping'][:, 0] = damp[:, 1]
-    sim = DynSim(m, N, table=t)
+    sim = EmuSim(m, N, table=t)
     sim.set_state(st)
     dt, g = m.param('dt'), np.array([0, 0, m.param('gravity_z')])
     v = st[:, f0 + 7:f0 + 10].astype(np.float64)
@@ -260,7 +260,7 @@ def test_free_flight_with_per_env_damping():
 
 # ------------------------------------------------------------------ randomization kernel
 def _rsim(m, N, counters, seed=77, env_offset=0):
-    sim = DynSim(m, N, table=model_table(m, N), seed=seed, env_offset=env_offset)
+    sim = EmuSim(m, N, table=model_table(m, N), seed=seed, env_offset=env_offset)
     o_cnt = Oracle(m).state_dim - 1
     sim.state[:, o_cnt] = counters
     return sim

@@ -160,11 +160,9 @@ def test_emu_records_read_in_place_when_stage_is_small():
     """Capacity only costs speed, never contacts: with tiny solver stages (arm-island classes of 104-120 q, free-body
     stage of 16 q) every grasp lands in the last class and most of its records are read from the class buffer in
     place; the grasp sequence must give the SAME states as the normal build, bit for bit."""
-    from emu_lib import lib_variant
     from helpers import SMALL_STAGE
-    small = lib_variant('smallstage', SMALL_STAGE)
     m = load_model('UR5PlayAbsRPY1Obj-v0')
-    a_sim, b_sim, o = EmuSim(m, 1, seed=3), EmuSim(m, 1, seed=3, library=small), Oracle(m, seed=3)
+    a_sim, b_sim, o = EmuSim(m, 1, seed=3), EmuSim(m, 1, seed=3, tag='smallstage', defines=SMALL_STAGE), Oracle(m, seed=3)
     o.reset()
     blk = o.state[60:63].copy()
     act = lambda z, g: np.array([blk[0], blk[1], z, 0, 0, 0, g])

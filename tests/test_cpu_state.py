@@ -10,8 +10,10 @@ import numpy as np
 import pytest
 
 import emu_arm
+import emu_lib
 import emu_state as S
 import np_arm_dynamics as R
+from emu_lib import EmuSim
 from np_state import host_edit as _host_edit, normalised as _normalised, quat_mat as _quat_mat, reference_rows
 from helpers import random_actions
 from oracle.oracle import Oracle
@@ -61,7 +63,7 @@ def _check_reads(m, sim, tag):
 
 def _oracle_reset_sim(env_id, n, seed):
     m = load_model(env_id)
-    s = S.sim(m, n)
+    s = EmuSim(m, n)
     for i in range(n):
         o = Oracle(m, seed=seed + i)
         o.reset()
@@ -71,7 +73,7 @@ def _oracle_reset_sim(env_id, n, seed):
 
 def _stepped(env_id, n, seed, steps=6):
     m = load_model(env_id)
-    s = S.sim(m, n, seed=seed)
+    s = EmuSim(m, n, seed=seed)
     s.reset()
     rng = np.random.default_rng(seed)
     for _ in range(steps):
@@ -92,7 +94,7 @@ def test_reads_match_reference_reset_and_stepped_states(env_id):
 def test_reads_match_reference_golden_states(golden):
     st = np.load(os.path.join(GOLDEN, golden))['state'][:6]
     m = load_model(PLAY)
-    s = S.sim(m, len(st))
+    s = EmuSim(m, len(st))
     s.state[:, :s.state_dim] = st
     _check_reads(m, s, golden)
 
@@ -119,7 +121,7 @@ def test_link_points_and_com_velocity_agree_with_arm_dynamics(env_id):
 
 # ------------------------------------------------------------------ writes
 def _twin(s):
-    t = S.sim(s.m, s.N, seed=s.seed)
+    t = EmuSim(s.m, s.N, seed=s.seed)
     t.state[:] = s.state
     for k in s.out:
         t.out[k][:] = s.out[k]
@@ -279,7 +281,7 @@ def test_invalid_calls_are_rejected_before_any_launch():
     assert s.state.tobytes() == st0.tobytes()
     assert all(s.out[k].tobytes() == out0[k].tobytes() for k in out0)
     pick = load_model('pandaPick-v0')             # nd 9, one free body, no slide
-    p = S.sim(pick, 4)
+    p = EmuSim(pick, 4)
     with pytest.raises(ValueError, match='nd \\+ n_slide = 9'):
         S.write_state(p, W(1 << 9, 0, 0, 0, 0), np.zeros((4, 9)))
     with pytest.raises(ValueError, match='n_free = 1'):
@@ -301,7 +303,7 @@ def test_struct_layouts_match_c(tmp_path):
                    W.joint_velocities.offset, W.free_poses.offset, W.free_velocities.offset, W.reserved.offset]
     for name in ('prb_body_states', 'prb_write_state', 'prb_save_state', 'prb_restore_state'):
         assert name in lib.SYMBOLS
-    assert S.lib().semu_max_bodies() == 17
+    assert emu_lib.lib().emu_max_bodies() == 17
 
 
 def test_state_ids_and_python_checks():
