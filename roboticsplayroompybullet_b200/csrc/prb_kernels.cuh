@@ -890,7 +890,7 @@ PRB_D void phase_collide_narrow(const DevModel& M, WM& W, int lane) {
 #pragma unroll 1
   for (int h = 0; h * 32 < n_runs; h++) {
     const int r = h * 32 + lane;
-    int keep[4], m = 0;
+    int keep[4] = {0, 0, 0, 0}, m = 0;
     if (r < n_runs) {
       int b0 = W.ovl[r], b1 = (r + 1 < n_runs) ? (int)W.ovl[r + 1] : ncand;
       if (b0 > ncand) b0 = ncand;
@@ -919,9 +919,28 @@ PRB_D void phase_collide_narrow(const DevModel& M, WM& W, int lane) {
       }
     }
     int t2;
-    const int off2 = total2 + warp_excl_scan(m, lane, &t2);
+    const int first = warp_excl_scan(m, lane, &t2);     // this run's first output, relative to the pass
+    // Copy in order of destination, 32 destinations per trip: lane = destination, its source from the run that owns it
+    // (the last lane whose first output is <= it).  ct may be the head of cand (SetupMemT): a contact's source is never
+    // before its destination, so a trip's writes land only on sources of this or an earlier trip (read before the
+    // __syncwarp) and never on those of later trips or passes.  (Lanes that each wrote their own run's contacts could
+    // overwrite one that another lane of the pass has still to read.)
+#pragma unroll 1
+    for (int base = 0; base < t2 && total2 + base < WM::Cfg::MAXCONTACT; base += 32) {
+      const int rel = base + lane;
+      int own = 0;
+#pragma unroll
+      for (int s = 16; s > 0; s >>= 1) if (__shfl_sync(FULL, first, own + s) <= rel) own += s;
+      const int i = rel - __shfl_sync(FULL, first, own);
+      const int k0 = __shfl_sync(FULL, keep[0], own), k1 = __shfl_sync(FULL, keep[1], own);
+      const int k2 = __shfl_sync(FULL, keep[2], own), k3 = __shfl_sync(FULL, keep[3], own);
+      const int dst = total2 + rel, src = i == 0 ? k0 : (i == 1 ? k1 : (i == 2 ? k2 : k3));
+      Contact kc;
+      if (rel < t2 && dst < WM::Cfg::MAXCONTACT) kc = W.cand[src];
+      __syncwarp();
+      if (rel < t2 && dst < WM::Cfg::MAXCONTACT) W.ct[dst] = kc;
+    }
     total2 += t2;
-    for (int i = 0; i < m; i++) if (off2 + i < WM::Cfg::MAXCONTACT) W.ct[off2 + i] = W.cand[keep[i]];
   }
   if (lane == 0) {
     W.n_contact = total2 < WM::Cfg::MAXCONTACT ? total2 : WM::Cfg::MAXCONTACT;

@@ -225,7 +225,9 @@ struct SetupCfg {
 #define SETUP_ALIGN2() ((void)0)
 #endif
 
-// shared memory of one env in the setup kernel: state + the substep's kinematics / collision scratch
+// shared memory of one env in the setup kernel: state + the substep's kinematics / collision scratch.  2 blocks x 8 envs
+// per SM take 120 kB of the SM's 256 kB of L1 / shared memory and leave the rest to L1 (11 784 B per env before the
+// phases shared one region: 27.8 -> 23.9 ms of setup per env step, profiles/r3_setup_smem.md).
 template <class CFG>
 struct SetupMemT {
   typedef CFG Cfg;
@@ -236,20 +238,30 @@ struct SetupMemT {
   float lp[PRB_MAXD][3], la[PRB_MAXD][3], lc[PRB_MAXD][3], lw[PRB_MAXD][3], lv[PRB_MAXD][3];
   float fR[PRB_MAXFREE][9], fIinv[PRB_MAXFREE][6];
   float sp[PRB_MAXSLIDE][3], sR[PRB_MAXSLIDE][9];
-  float Minv[PRB_MAXD][PRB_MAXD + 1], Q[PRB_MAXD];
-  float vs[32];
+  float Minv[PRB_MAXD][PRB_MAXD + 1];
+  float vs[30];                                   // velocity DoF (nv <= 27); 30 keeps sizeof an odd multiple of 8 (below)
   float fdyn[PRB_MAXFREE * FD_N];                 // the env's free-body constants (phase_fk FD_* layout)
   const float* fric;                              // the env's collider friction row: the dynamics table's or the model's
   const float* spin;
   unsigned short ovl[CFG::MAXOVL];
-  int n_ovl, n_contact, n_jrow, pool_used, overflow;
+  int n_ovl, n_contact, n_jrow, overflow;
   int dbg_a, dbg_c, dbg_p, dbg_u;
-  Contact ct[CFG::MAXCONTACT];
-  float lR[PRB_MAXD][9], lIw[PRB_MAXD][6], lf[PRB_MAXD][3], ln[PRB_MAXD][3];
-  float Mm[PRB_MAXD][PRB_MAXD + 1];
-  float2 aabb[PRB_MAXCOL][3];     // per axis (lo, hi)
-  Contact cand[CFG::MAXCAND];
+  float lR[PRB_MAXD][9], lIw[PRB_MAXD][6], lf[PRB_MAXD][3], ln[PRB_MAXD][3];   // phase_fk (lR: also collider frames, observe)
+  // one region, reused by the phases in turn
+  union {
+    float2 aabb[PRB_MAXCOL][3];   // broad phase: per axis (lo, hi)
+    Contact cand[CFG::MAXCAND];   // narrow phase; manifold reduction compacts the kept contacts into its head: ct
+    struct {
+      Contact ct[CFG::MAXCONTACT];          // narrow phase -> phase_rows_stream
+      float Mm[PRB_MAXD][PRB_MAXD + 1];     // phase_crba -> phase_minv
+      float Q[PRB_MAXD];                    // phase_crba -> phase_vstar
+    };
+  };
 };
+static_assert(SetupCfg::MAXCONTACT <= SetupCfg::MAXCAND, "ct is the head of cand");
+// With a size that is a multiple of 16 every env's W is 16-byte aligned, ptxas merges shared loads into 128-bit ones
+// (230 LDS.128 instead of 63 in prb_setup_kernel<12>) and the kernel spills at its 128 registers.
+static_assert(sizeof(SetupMemT<SetupCfg>) % 16 == 8, "setup kernel shared memory per env: keep W 8-byte aligned only");
 
 PRB_D int body_kind(const DevModel& M, int body) { return body < 0 ? K_STATIC : (body == 0 ? K_ARM : (body <= M.n_free ? K_FREE : K_SLIDE)); }
 PRB_D int kind_rank(int k) { return k == K_ARM ? 3 : (k == K_SLIDE ? 2 : (k == K_FREE ? 1 : 0)); }
